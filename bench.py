@@ -25,6 +25,10 @@ Workload (BASELINE.json configs[1]): a synthetic replica of chignolin (cln025: 1
 package made by `oracle/make_ref.py`, behind the exact-solve `qpsolvers` stand-in) on a bounded frame
 sample with all host threads; the float64 numpy port in `oracle/` is the fallback when the copy is
 absent.
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's share) as `DIR/<name>.npy`, so
+that two builds can be compared output for output on the same seeded inputs: the constraint set, both
+fitted force maps and residuals, and the four mapped arrays on a fixed sample of frames (`frames.npy`).
 """
 from __future__ import annotations
 
@@ -41,17 +45,28 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
 
 METRIC = "frames/sec through force-map fit+apply"
 UNIT = "frames/s"
 L2_REG = 1e3
 KBT = 0.6955215
+# frames of each mapped array written by --dump-outputs: 4 arrays x 32 768 frames x 10 beads x 3 x 8 B = 31 MB
+DUMP_FRAMES = 32_768
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def _at_least_one(text: str) -> int:
+    n = int(text)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {n}")
+    return n
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=_at_least_one, default=5, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--frames", type=int, default=1_000_000, help="frames per GPU")
@@ -59,7 +74,12 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the config 3/4/5 probes")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the outputs of the last timed step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 # ----------------------------------------------------------------------------- CPU arm
@@ -145,6 +165,32 @@ def workload_config(frames_per_gpu: int) -> dict:
         "frames_per_gpu": frames_per_gpu,
         "cache": "inputs (2.1 GB per array per GPU) are larger than L2; no explicit flush",
     }
+
+
+def step_outputs(cons, r_uni, r_opt, n_frames: int) -> dict:
+    """What one step hands its caller, as host float32 / float64 arrays: the constraint set (sorted site
+    pairs), each map's force matrix and residual, and the mapped arrays on a fixed, seeded sample of frames."""
+    import torch
+
+    frames = np.sort(np.random.default_rng(0).choice(n_frames, size=min(n_frames, DUMP_FRAMES), replace=False))
+    out = {"frames": frames.astype(np.float64),
+           "constraints": np.array(sorted(sorted(p) for p in cons), dtype=np.float64).reshape(-1, 2)}
+    for tag, res in (("uni", r_uni), ("opt", r_opt)):
+        out[f"{tag}_force_map"] = np.asarray(res["tmap"].force_map.standard_matrix, dtype=np.float64)
+        out[f"{tag}_residual"] = np.array([res["residual"]], dtype=np.float64)
+        for key in ("mapped_coords", "mapped_forces"):
+            arr = torch.as_tensor(res[key])
+            sample = arr.index_select(0, torch.as_tensor(frames, device=arr.device)).cpu().numpy()
+            out[f"{tag}_{key}"] = sample if sample.dtype == np.float32 else sample.astype(np.float64)
+    return out
+
+
+def dump_outputs(outputs: dict, where: Path) -> None:
+    total = sum(a.nbytes for a in outputs.values())
+    assert total <= DUMP_LIMIT_BYTES, f"--dump-outputs would write {total} bytes"
+    where.mkdir(parents=True, exist_ok=True)
+    for name, arr in outputs.items():
+        np.save(where / f"{name}.npy", arr)
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -357,8 +403,9 @@ def main() -> None:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         n0 = _lib.LAUNCHES["count"]
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()  # what the last timed step returned (earlier results are dropped as they come)
         e1.record()
         barrier()
         launches = _lib.LAUNCHES["count"] - n0
@@ -374,7 +421,7 @@ def main() -> None:
                    and time.perf_counter() - t_a < 1.0):
                 fn()
             clocks = sampler.stop()
-        return float(ms.item()) / steps, launches, clocks
+        return float(ms.item()) / steps, launches, clocks, last
 
     def kernel_times(fn):
         """{entry point: [ms per call]} of one extra pass (CUDA events on the launching stream)."""
@@ -397,7 +444,11 @@ def main() -> None:
     ctx = agf.frame_sharding(world > 1)
     with ctx:
         # ---- device-resident throughput
-        ms_dev, launches, clocks = timed(lambda: step(coords, forces), args.steps, args.warmup, sample_clocks=True)
+        ms_dev, launches, clocks, last = timed(lambda: step(coords, forces), args.steps, args.warmup,
+                                               sample_clocks=True)
+        if args.dump_outputs is not None and rank == 0:
+            dump_outputs(step_outputs(*last, T), args.dump_outputs)
+        del last
         per_kernel = kernel_times(lambda: step(coords, forces))
 
         # ---- end to end from pinned host memory
@@ -416,14 +467,14 @@ def main() -> None:
                 _, r1, r2 = step(c, f)
                 d2h["n"] = sum(r[k].nbytes for r in (r1, r2) for k in ("mapped_coords", "mapped_forces"))
 
-            ms_e2e, _, _ = timed(host_step, max(1, min(args.steps, 5)), 3)
+            ms_e2e, _, _, _ = timed(host_step, args.steps, 3)
             # what the host side can deliver: all ranks upload their pinned coordinate array at once
             dst = torch.empty_like(coords)
 
             def upload():
                 dst.copy_(hc, non_blocking=True)
 
-            ms_up, _, _ = timed(upload, 3, 1)
+            ms_up, _, _, _ = timed(upload, 3, 1)
             h2d_probe = world * hc.numel() * 4 / (ms_up * 1e-3) / 1e9
             del dst
             moved = int(nc.nbytes + nf.nbytes)

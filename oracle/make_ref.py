@@ -1,11 +1,11 @@
 """Recipe for ``oracle/_ref``: a runnable copy of the reference's own Python package.
 
-TEST / BENCH INFRASTRUCTURE ONLY.  ``python oracle/make_ref.py`` (called by
-``__graft_entry__.build()`` when ``/root/reference`` is present, i.e. in the build container)
-copies ``/root/reference/src/aggforce`` UNMODIFIED into ``oracle/_ref/aggforce``.  ``oracle/_ref/``
-is git-ignored (reference sources never enter the history) but travels to the GPU box with the
-snapshot, where ``bench.py --impl reference`` and ``bench.py``'s ``cpu_baseline`` leg time the
-reference's own ``guess_pairwise_constraints`` / ``project_forces`` on the host cores.
+TEST / BENCH INFRASTRUCTURE ONLY.  ``python oracle/make_ref.py <reference checkout>`` copies
+``<reference checkout>/src/aggforce`` UNMODIFIED into ``oracle/_ref/aggforce``.  ``oracle/_ref/``
+is git-ignored (reference sources never enter the history); where it exists, ``bench.py --impl
+reference`` and ``bench.py``'s ``cpu_baseline`` leg time the reference's own
+``guess_pairwise_constraints`` / ``project_forces`` on the host cores, and where it does not they
+time the numpy port in ``oracle/``.
 
 The reference imports ``qpsolvers`` (absent here, unpinned in its ``setup.cfg``); ``load()`` installs
 ``oracle/qpsolvers_shim.py`` -- the exact equality-QP solve -- under that name before importing it.
@@ -19,20 +19,20 @@ import sys
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
-REF_SRC = Path("/root/reference/src/aggforce")
 DEST = HERE / "_ref"
 
 
-def make() -> Path | None:
-    """Copy the reference package; returns the destination or ``None`` when the mount is absent."""
-    if not REF_SRC.is_dir():
-        return None
+def make(reference: str | Path) -> Path:
+    """Copy the package ``<reference>/src/aggforce`` of a reference checkout; returns the destination."""
+    src = Path(reference) / "src" / "aggforce"
+    if not src.is_dir():
+        raise FileNotFoundError(f"{src} is not a directory: pass the root of an aggforce checkout")
     if DEST.exists():
         shutil.rmtree(DEST)
     DEST.mkdir(parents=True)
-    shutil.copytree(REF_SRC, DEST / "aggforce", ignore=shutil.ignore_patterns("__pycache__", "*.pyc"))
+    shutil.copytree(src, DEST / "aggforce", ignore=shutil.ignore_patterns("__pycache__", "*.pyc"))
     (DEST / "README").write_text(
-        "Unmodified copy of /root/reference/src/aggforce made by oracle/make_ref.py; git-ignored, not product.\n")
+        "Unmodified copy of the reference's src/aggforce made by oracle/make_ref.py; git-ignored, not product.\n")
     return DEST
 
 
@@ -57,4 +57,6 @@ def load():
 
 
 if __name__ == "__main__":
-    print(make())
+    if len(sys.argv) != 2:
+        sys.exit("usage: python oracle/make_ref.py <reference checkout>")
+    print(make(sys.argv[1]))
