@@ -976,9 +976,11 @@ def pair_constraints(frames: Frames, other: Optional[Frames], threshold: float):
     world = _dist().get_world_size(_Sharding.group) if sharded() else 1
 
     def other_piece(piece_t0: int, count: int) -> Optional[torch.Tensor]:
+        # the frames matching a piece of `frames`: a host cross array too large to keep resident is
+        # uploaded range by range, as `frames` itself is
         if other is None:
             return None
-        return other.resident()[piece_t0 : piece_t0 + count]
+        return other.frame_range(piece_t0, count)
 
     # ---- stage 0: literal all-pairs pass over a short prefix
     n0 = _screen_frames(float(t_total if t_total is not None else world * t_local), float(threshold), t_local)

@@ -254,6 +254,7 @@ static int pair_moments_typed(const void* xyz, const void* other, int64_t n_fram
                               const int32_t* pairs, int64_t n_pairs, const double* shift, double* acc,
                               cudaStream_t stream) {
   constexpr int KF = sizeof(T) == 4 ? 16 : 8;
+  // the pairs are listed explicitly, so other == xyz (the same data) may take the self-mode ring
   const bool self = (other == nullptr || other == xyz);
   size_t stage_bytes = ((size_t)KF * n_sites * 3 * sizeof(T) + 15) / 16 * 16;
   size_t smem = 128 + kPairStages * stage_bytes;
@@ -319,7 +320,7 @@ extern "C" int agf_pair_first(const void* xyz, const void* other, int dtype, int
   AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_pair_first: bad dtype");
   if (n_pairs == 0) return AGF_OK;
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const bool self = (other == nullptr || other == xyz);
+  const bool self = (other == nullptr || other == xyz);  // explicit pair list: the same array reads the same
   int blocks = (int)((n_pairs + 255) / 256);
   if (dtype == AGF_F32)
     pair_first_kernel<float><<<blocks, 256, 0, s>>>(reinterpret_cast<const float*>(xyz),
@@ -340,7 +341,9 @@ extern "C" int agf_pair_screen(const void* xyz, const void* other, int dtype, in
   AGF_REQUIRE(n_frames > 0 && n_sites > 0, "agf_pair_screen: bad sizes");
   AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_pair_screen: bad dtype");
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const bool self = (other == nullptr || other == xyz);
+  // self mode is other == NULL only: the same array passed as `other` is a cross-mode request, which
+  // also visits the diagonal and both orders of every pair
+  const bool self = other == nullptr;
   const int n_o = self ? n_sites : n_other;
   const int n_jb = (n_sites + 31) / 32;
   dim3 grid(n_jb < 8 ? n_jb : 8, n_o);  // up to eight blocks per row share its column blocks
@@ -363,7 +366,7 @@ extern "C" int agf_pair_select(const double* m2, double bound, const double* cou
   using namespace agf;
   AGF_REQUIRE(m2 && xyz && pairs && shift && acc && count, "agf_pair_select: null pointer");
   AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_pair_select: bad dtype");
-  const bool self = (other == nullptr || other == xyz);
+  const bool self = other == nullptr;  // as in agf_pair_screen: the same array as `other` is cross mode
   const int n_o = self ? n_sites : n_other;
   AGF_REQUIRE(n_sites > 0 && n_o > 0 && cap > 0 && (int64_t)n_sites * n_o <= (1 << 18),
               "agf_pair_select: at most 2^18 candidate pairs (got %d x %d)", n_o, n_sites);

@@ -14,6 +14,7 @@ import numpy as np
 
 __all__ = [
     "pair_distance_sd",
+    "pair_distance_moments",
     "guess_pairwise_constraints",
     "guess_pairwise_constraints_literal",
     "merge_constraint_groups",
@@ -74,6 +75,27 @@ def pair_distance_sd(xyz: np.ndarray, cross_xyz: Optional[np.ndarray] = None) ->
         dev = np.sqrt((d * d).sum(-1)) - mean
         m2 += (dev * dev).sum(0)
     return np.sqrt(m2 / n_frames)
+
+
+def pair_distance_moments(xyz: np.ndarray, other: Optional[np.ndarray], pairs: np.ndarray,
+                          shift: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
+    """Per-pair shifted moments ``(sum_t e_t, sum_t e_t**2)`` with ``e_t = d_t - shift[p]`` and
+    ``d_t = |xyz[t, j] - other[t, i]|`` for ``pairs[p] = (i over other, j over xyz)``, in float64.
+
+    ``other=None`` is the self case.  This is what kernel (c) accumulates for a pair list; with it
+    ``pair_distance_sd`` of a listed pair is ``sqrt((s2 - s1**2 / T) / T)``."""
+    x = np.asarray(xyz, dtype=np.float64)
+    o = x if other is None else np.asarray(other, dtype=np.float64)
+    p = np.asarray(pairs, dtype=np.int64).reshape(-1, 2)
+    c = np.asarray(shift, dtype=np.float64).reshape(-1)
+    s1, s2 = np.zeros(len(p)), np.zeros(len(p))
+    block = max(1, int(4e6 // max(1, 3 * len(p))))
+    for s in range(0, x.shape[0], block):
+        d = x[s : s + block, p[:, 1]] - o[s : s + block, p[:, 0]]
+        e = np.sqrt((d * d).sum(-1)) - c
+        s1 += e.sum(0)
+        s2 += (e * e).sum(0)
+    return s1, s2
 
 
 def guess_pairwise_constraints(

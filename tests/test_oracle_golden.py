@@ -25,6 +25,33 @@ def test_pair_sd_and_constraint_sets(small_cln):
     assert len(cross) > 0
 
 
+@pytest.mark.parametrize("cross", [False, True])
+def test_pair_distance_moments_give_pair_distance_sd(small_cln, cross):
+    """The per-pair moments (the quantity kernel (c) accumulates) reproduce pair_distance_sd on a pair
+    list, for any shift: a shift only moves the moments, not the variance they imply."""
+    coords = small_cln["coords"][:, :60]
+    other = small_cln["coords"][:, 40:90] if cross else None
+    sds = oracle.pair_distance_sd(coords, other)
+    rng = np.random.default_rng(0)
+    ii, jj = np.nonzero(np.ones_like(sds))
+    pick = rng.choice(ii.size, 300, replace=False)
+    pairs = np.stack([ii[pick], jj[pick]], axis=1)
+    o = coords if other is None else other
+    frame0 = np.linalg.norm(coords[0, pairs[:, 1]].astype(np.float64) - o[0, pairs[:, 0]], axis=-1)
+    T = coords.shape[0]
+    for shift in (frame0, np.zeros(len(pairs)), frame0 + rng.normal(0, 0.1, len(pairs))):
+        s1, s2 = oracle.pair_distance_moments(coords, other, pairs, shift)
+        assert s1.shape == s2.shape == (len(pairs),)
+        # M2 = s2 - s1^2 / T loses what the shift leaves of the mean: compare on the scale of s2
+        m2_ref = T * sds[pairs[:, 0], pairs[:, 1]] ** 2
+        assert np.all(np.abs((s2 - s1 * s1 / T) - m2_ref) <= 1e-12 * s2 + 1e-300)
+    # by definition: sum of e and of e^2 over frames
+    d = np.linalg.norm(coords[:, pairs[:3, 1]].astype(np.float64) - o[:, pairs[:3, 0]], axis=-1)
+    s1, s2 = oracle.pair_distance_moments(coords, other, pairs[:3], frame0[:3])
+    assert np.allclose(s1, (d - frame0[:3]).sum(0), rtol=1e-13, atol=1e-13)
+    assert np.allclose(s2, ((d - frame0[:3]) ** 2).sum(0), rtol=1e-13, atol=1e-16)
+
+
 def test_constraints_are_the_xh_bonds(small_cln):
     from aggforce_b200.synth import chignolin_topology
 
