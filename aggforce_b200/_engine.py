@@ -395,6 +395,59 @@ def allgather_host(arr: np.ndarray) -> List[np.ndarray]:
     return [o.cpu().numpy() for o in outs]
 
 
+_CHECKED_WEIGHTS: dict = {}  # id -> weakref of device weight tensors this module made and validated
+
+
+def frame_weights_dev(frame_weights, n_frames: int) -> Optional[torch.Tensor]:
+    """Per-frame weights of a fit as a validated float64 device tensor (``None`` stays ``None``).
+
+    ``frame_weights``: 1-D numpy array or tensor, one entry per frame of this rank's slice, any float dtype.
+    Raises ``ValueError`` for a wrong length, a negative or non-finite entry, or a sum of zero -- under
+    ``frame_sharding`` the global sum, and every rank raises when any rank's slice is invalid (one exchange).
+    A tensor returned here is recognised when it is passed again (``project_forces`` forwards it to the
+    method), so the weights are uploaded and checked once per call."""
+    import weakref
+
+    if frame_weights is None:
+        return None
+    ref = _CHECKED_WEIGHTS.get(id(frame_weights))
+    if ref is not None and ref() is frame_weights and frame_weights.shape[0] == n_frames:
+        return frame_weights
+    if isinstance(frame_weights, torch.Tensor):
+        w = frame_weights.detach().to(device=device(), dtype=torch.float64).contiguous()
+    else:
+        arr = np.asarray(frame_weights)
+        if not (np.issubdtype(arr.dtype, np.floating) or np.issubdtype(arr.dtype, np.integer)):
+            raise ValueError(f"frame_weights must be a float array; got dtype {arr.dtype}")
+        w = torch.as_tensor(np.ascontiguousarray(arr, dtype=np.float64), device=device())
+    good_shape = w.dim() == 1 and int(w.shape[0]) == int(n_frames)
+    if good_shape:
+        bad = (~torch.isfinite(w) | (w < 0)).any().to(torch.float64)
+        local = torch.stack([bad, torch.where(bad > 0, torch.zeros_like(bad), w.sum())])
+    else:
+        local = torch.tensor([1.0, 0.0], dtype=torch.float64, device=device())
+    if sharded():
+        dist = _dist()
+        if dist.get_backend(_Sharding.group) != "nccl":
+            local = local.cpu()
+        dist.all_reduce(local, group=_Sharding.group)
+    n_bad, total = (float(v) for v in to_host(local.to(device())))
+    if not good_shape:
+        raise ValueError(f"frame_weights must be a 1-D array with one weight per frame ({n_frames}); "
+                         f"got shape {tuple(w.shape)}")
+    if n_bad > 0:
+        if sharded():
+            raise ValueError("frame_weights of some rank have a wrong length or a negative or non-finite entry")
+        raise ValueError("frame_weights must be finite and non-negative")
+    if not total > 0.0:
+        raise ValueError("frame_weights sum to zero" + (" over all ranks" if sharded() else ""))
+    if len(_CHECKED_WEIGHTS) > 64:
+        _CHECKED_WEIGHTS.clear()
+    if w is not frame_weights:
+        _CHECKED_WEIGHTS[id(w)] = weakref.ref(w)
+    return w
+
+
 def global_count(local: int) -> int:
     if not sharded():
         return int(local)
@@ -700,16 +753,26 @@ class GramPlan:
             self.slot_members |= (int(members.max()) if members.size else 1) << (8 * c)
 
 
-def gram_linear_raw(frames: Frames, col_of_site: np.ndarray, n_red: int,
-                    plan: Optional[GramPlan] = None) -> Tuple[torch.Tensor, np.ndarray]:
+def gram_linear_raw(frames: Frames, col_of_site: np.ndarray, n_red: int, plan: Optional[GramPlan] = None,
+                    weights: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, np.ndarray]:
     """Kernel (a): accumulated and all-reduced second-moment matrix as the kernels leave it --
     ``(gram f64 [n_red, n_red] with the element-wise UPPER triangle valid, order)`` where
-    ``order[p]`` is the caller's column held at internal position ``p``."""
+    ``order[p]`` is the caller's column held at internal position ``p``.  ``weights``: per-frame weights
+    from :func:`frame_weights_dev`; the weighted Gram runs on the FP64 DMMA kernels (the int8 paths
+    take their column scales from a sample of frames, which a heavy frame outside it would defeat)."""
     if plan is None:
         plan = GramPlan(col_of_site, n_red, want_i8=_GRAM_I8[0] and frames.np_dtype == np.float32)
     d_ptr, d_sites, order = plan.d_ptr, plan.d_sites, plan.order
     gram = torch.zeros((n_red, n_red), dtype=torch.float64, device=device())
-    for _, piece in frames.pieces():
+    for t0, piece in frames.pieces():
+        if weights is not None:
+            w = weights[t0 : t0 + piece.shape[0]]
+            need = int(_lib.lib().agf_gram_linear_workspace_bytes(frames.n_sites, n_red, piece.shape[0]))
+            ws = workspace(need) if need > 0 else None
+            _lib.call("agf_gram_linear_ws_weighted", ptr(piece), dtype_code(piece), piece.shape[0], frames.n_sites,
+                      ptr(d_ptr), ptr(d_sites), n_red, ptr(gram), ptr(ws), C.c_size_t(0 if ws is None else ws.numel()),
+                      ptr(w), stream_ptr())
+            continue
         need_i8 = 0
         if (_GRAM_I8[0] and plan.i8_shape and piece.dtype == torch.float32
                 and piece.shape[0] >= _GRAM_I8_MIN_FRAMES):
@@ -740,10 +803,11 @@ def gram_linear_raw(frames: Frames, col_of_site: np.ndarray, n_red: int,
     return gram, order
 
 
-def gram_linear(frames: Frames, col_of_site: np.ndarray, n_red: int) -> torch.Tensor:
+def gram_linear(frames: Frames, col_of_site: np.ndarray, n_red: int,
+                weights: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Kernel (a): all-reduced, symmetrised second-moment matrix (device f64 [n_red, n_red]) in the
-    caller's column order."""
-    gram, order = gram_linear_raw(frames, col_of_site, n_red)
+    caller's column order (``weights``: see :func:`gram_linear_raw`)."""
+    gram, order = gram_linear_raw(frames, col_of_site, n_red, weights=weights)
     _lib.call("agf_symmetrize", ptr(gram), n_red, stream_ptr())
     if not np.array_equal(order, np.arange(n_red)):
         rank = np.empty(n_red, dtype=np.int64)
@@ -751,6 +815,13 @@ def gram_linear(frames: Frames, col_of_site: np.ndarray, n_red: int) -> torch.Te
         back = _dev_cached(np.ascontiguousarray(rank, dtype=np.int64))  # cached: no pageable upload per call
         gram = gram[back][:, back]
     return gram
+
+
+def weighted_sumsq(x: torch.Tensor, weights: torch.Tensor, out: torch.Tensor) -> None:
+    """``out`` (device f64 [1], +=) gets ``sum_t weights[t] * sum(x[t]**2)`` of a device array ``(T, ...)``."""
+    x = x.contiguous()
+    _lib.call("agf_weighted_sumsq", ptr(x), dtype_code(x), x.shape[0], int(np.prod(x.shape[1:])), ptr(weights),
+              ptr(out), stream_ptr())
 
 
 class CompiledMap:

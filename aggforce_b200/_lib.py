@@ -22,6 +22,9 @@ _vp, _i32, _i64, _u64, _dbl, _flt = C.c_void_p, C.c_int32, C.c_int64, C.c_uint64
 SIGNATURES = {
     "agf_gram_linear": [_vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _vp, _vp],
     "agf_gram_linear_ws": [_vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _vp, _vp, C.c_size_t, _vp],
+    "agf_gram_linear_weighted": [_vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _vp, _vp, _vp],
+    "agf_gram_linear_ws_weighted": [_vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _vp, _vp, C.c_size_t, _vp, _vp],
+    "agf_weighted_sumsq": [_vp, C.c_int, _i64, _i32, _vp, _vp, _vp],
     "agf_gram_linear_i8": [_vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _i32, C.c_uint32, _vp, _vp, C.c_size_t, _vp],
     "agf_gram_linear_i8t": [_vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _vp, _vp, C.c_size_t, _vp],
     "agf_symmetrize": [_vp, _i32, _vp],
@@ -42,6 +45,10 @@ SIGNATURES = {
                       _dbl, _vp, _vp],
     "agf_gram_feat_ws": [_vp, _vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _i32, _dbl,
                          _dbl, _dbl, _vp, _vp, C.c_size_t, _vp],
+    "agf_gram_feat_weighted": [_vp, _vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _i32,
+                               _dbl, _dbl, _dbl, _vp, _vp, _vp],
+    "agf_gram_feat_ws_weighted": [_vp, _vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _i32,
+                                  _dbl, _dbl, _dbl, _vp, _vp, C.c_size_t, _vp, _vp],
     "agf_gram_feat_i8": [_vp, _vp, C.c_int, _i64, _i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _i32, _dbl,
                          _dbl, _dbl, _vp, _vp, C.c_size_t, _vp],
     "agf_symmetrize_batch": [_vp, _i32, _i32, _vp],

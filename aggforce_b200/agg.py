@@ -48,6 +48,18 @@ def _global_mean_sq(sumsq: float, shape) -> float:
     return float(tot[0] / tot[1])
 
 
+def _weighted_residual(mapped_forces, weights: torch.Tensor) -> float:
+    """``sum_t w_t sum F_t**2 / (size of one frame * sum_t w_t)`` over all ranks (maps applied as a whole)."""
+    dev = mapped_forces if isinstance(mapped_forces, torch.Tensor) else torch.as_tensor(mapped_forces)
+    dev = dev.to(_engine.device())
+    num = torch.zeros(1, dtype=torch.float64, device=dev.device)
+    _engine.weighted_sumsq(dev, weights, num)
+    per_frame = float(np.prod(tuple(dev.shape[1:])))
+    local = _engine.to_host(torch.cat([num, (weights.sum() * per_frame).reshape(1)]))
+    tot = np.sum(_engine.allgather_host(local), axis=0)
+    return float(tot[0] / tot[1])
+
+
 def project_forces(
     coords,
     forces,
@@ -66,6 +78,15 @@ def project_forces(
 
     Returns a dict with keys ``mapped_coords``, ``mapped_forces``, ``tmap``, ``residual``
     (mean squared mapped force, not held out) and ``constraints``.
+
+    ``frame_weights`` (extension, keyword): one non-negative weight per frame (numpy or CUDA tensor; under
+    ``frame_sharding`` the weights of this rank's frames), for trajectories that are not samples of the
+    target ensemble (reweighted biased runs, pooled or bootstrapped datasets).  It is forwarded to
+    ``method`` (``qp_linear_map`` and ``qp_feat_linear_map`` fit the weighted objective,
+    ``constraint_aware_uni_map`` ignores it) and the residual becomes the weighted mean
+    ``sum_t w_t sum F_t**2 / (3 n_cg sum_t w_t)``.  ``mapped_coords`` / ``mapped_forces`` are the per-frame
+    mapped arrays as without weights.  Constraint detection (``constrained_inds="auto"``) stays
+    unweighted: a rigid pair is rigid in every frame, whatever its weight.
     """
     auto = isinstance(constrained_inds, str) and constrained_inds == PROJECT_FORCES_CNSTR_AUTO
     if auto and coords is None:
@@ -80,6 +101,9 @@ def project_forces(
 
 def _project_forces(t, coords, forces, coord_map, constrained_inds, auto, method, kwargs) -> Dict[str, Any]:
     coords_in, forces_in = _engine.Frames(coords), _engine.Frames(forces)
+    weights = _engine.frame_weights_dev(kwargs.get("frame_weights"), forces_in.n_frames)
+    if weights is not None:
+        kwargs = dict(kwargs, frame_weights=weights)  # checked and uploaded once: the method reuses it
     if auto:
         constrained_inds = guess_pairwise_constraints(coords_in)
     # ONE status buffer for both applications: [sum(out_c^2), sum(out_f^2), n_elements, flags_c, flags_f]
@@ -128,22 +152,26 @@ def _project_forces(t, coords, forces, coord_map, constrained_inds, auto, method
                 stat.zero_()
         _engine.run_deferred()
         fc, oc, _ = early["launch"] if "launch" in early else cm._launch(coords_in, slots=slots_c, download=dl_c)
-        ff, of, _ = fm._launch(forces_in, want_sumsq=True, slots=slots_f, download=dl_f)
+        ff, of, _ = fm._launch(forces_in, want_sumsq=weights is None, slots=slots_f, download=dl_f)
         host_c = dl_c[0] if dl_c else None  # downloads overlap the force upload, piece by piece
         host_f = dl_f[0] if dl_f else None
         pend = fm._pending if fm._matrix is None else None
         n_elem = float(np.prod(of.shape))
+        if weights is not None:  # weighted residual: numerator and denominator 3 n_cg sum(w) in the same slots
+            _engine.weighted_sumsq(of, weights, stat[1:2])
+            stat[2:3].copy_((weights.sum() * float(np.prod(of.shape[1:]))).reshape(1))
         if _engine.sharded():
             # residual numerator / denominator are summed over ranks and the NaN flags max-ed, so that a
             # violated NaN protocol raises on every rank (a lone raiser would leave the others in the next
             # collective): ONE message
-            stat[2:3].copy_(_engine.dev_f64([n_elem]))
+            if weights is None:
+                stat[2:3].copy_(_engine.dev_f64([n_elem]))
             _engine.allreduce_sum_max_(stat, 3)
         if pend is not None and pend.buf is None:
             pend = None  # a large device fit: checked when it was solved, downloaded only on request
         got = _engine.read_many([stat] + ([pend.buf] if pend is not None else []))
         st = got[0]
-        if _engine.sharded():
+        if _engine.sharded() or weights is not None:
             n_elem = float(st[2])
         status = np.array([st[0], st[1], st[3], st[4]])
         if pend is not None:
@@ -157,7 +185,11 @@ def _project_forces(t, coords, forces, coord_map, constrained_inds, auto, method
             traj_map = SeperableTMap(coord_map=cm, force_map=fm)
             mapped_coords = cm._finish(fc, oc, status[2:3], host_c)
             mapped_forces = fm(forces_in)
-            residual = _global_mean_sq(float((torch.as_tensor(mapped_forces).double() ** 2).sum()), mapped_forces.shape)
+            if weights is not None:
+                residual = _weighted_residual(mapped_forces, weights)
+            else:
+                residual = _global_mean_sq(float((torch.as_tensor(mapped_forces).double() ** 2).sum()),
+                                           mapped_forces.shape)
         else:
             mapped_coords = cm._finish(fc, oc, status[2:3], host_c)
             mapped_forces = fm._finish(ff, of, status[3:4], host_f)
@@ -166,7 +198,7 @@ def _project_forces(t, coords, forces, coord_map, constrained_inds, auto, method
         _engine.clear_deferred()
         mapped = traj_map(t)
         mapped_coords, mapped_forces = mapped.coords, mapped.forces
-        residual = force_smoothness(mapped_forces)
+        residual = force_smoothness(mapped_forces) if weights is None else _weighted_residual(mapped_forces, weights)
     return {
         PROJCOORDS_KNAME: mapped_coords,
         PROJFORCES_KNAME: mapped_forces,
@@ -196,7 +228,13 @@ def project_forces_grid_cv(
     is ``trace(W G_fold W') / (3 T_fold n_cg)`` -- no further pass over the frames for any grid
     point.  Everything else runs ``project_forces`` per fold and grid point as the reference does
     (it calls ``tmap.from_arrays``, which no TMap defines; ``map_arrays`` is used here).
+
+    ``frame_weights`` are not supported here: per-fold fits would need the weights of each fold's frames.
+    Passing them raises ``ValueError``.
     """
+    if kwargs.get("frame_weights") is not None:
+        raise ValueError("project_forces_grid_cv does not take frame_weights: the full-length weights do not match "
+                         "the frames of a fold's fit")
     n_frames = forces.shape[0]
     frames = np.arange(n_frames)
     (np.random.default_rng() if rng is None else rng).shuffle(frames)

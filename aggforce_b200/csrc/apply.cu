@@ -973,3 +973,54 @@ extern "C" int agf_map_apply_slice(const void* points, int in_dtype, int64_t n_f
   AGF_CUDA_TRY(cudaGetLastError());
   return AGF_OK;
 }
+
+// ------------------------------------------------------------------ weighted residual
+// sumsq += sum_t w_t sum_e x[t, e]^2 over a mapped array [n_frames, per_frame]: warp = frame, lanes stride its
+// elements; one float64 atomic per block.
+namespace agf {
+template <typename T>
+__global__ void __launch_bounds__(256) weighted_sumsq_kernel(const T* __restrict__ x, int64_t n_frames, int per_frame,
+                                                             const double* __restrict__ w, double* sumsq) {
+  __shared__ double s_part[8];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  double acc = 0.0;
+  for (int64_t t = (int64_t)blockIdx.x * 8 + warp; t < n_frames; t += (int64_t)gridDim.x * 8) {
+    const T* row = x + t * per_frame;
+    double s = 0.0;
+    for (int e = lane; e < per_frame; e += 32) {
+      const double v = to_f64(row[e]);
+      s += v * v;
+    }
+    acc += __ldg(w + t) * s;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if (lane == 0) s_part[warp] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double b = 0.0;
+    for (int i = 0; i < 8; ++i) b += s_part[i];
+    atomicAdd(sumsq, b);
+  }
+}
+}  // namespace agf
+
+extern "C" int agf_weighted_sumsq(const void* x, int dtype, int64_t n_frames, int32_t per_frame,
+                                  const double* frame_weights, double* sumsq, void* stream) {
+  using namespace agf;
+  AGF_REQUIRE(x && frame_weights && sumsq, "agf_weighted_sumsq: null pointer");
+  AGF_REQUIRE(n_frames >= 0 && per_frame > 0, "agf_weighted_sumsq: bad sizes");
+  AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_weighted_sumsq: bad dtype");
+  if (n_frames == 0) return AGF_OK;
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const int64_t want = (n_frames + 7) / 8;
+  const int blocks = (int)(want < (int64_t)sm_count() * 8 ? want : (int64_t)sm_count() * 8);
+  if (dtype == AGF_F32)
+    weighted_sumsq_kernel<float><<<blocks, 256, 0, s>>>(reinterpret_cast<const float*>(x), n_frames, per_frame,
+                                                        frame_weights, sumsq);
+  else
+    weighted_sumsq_kernel<double><<<blocks, 256, 0, s>>>(reinterpret_cast<const double*>(x), n_frames, per_frame,
+                                                         frame_weights, sumsq);
+  AGF_CUDA_TRY(cudaGetLastError());
+  return AGF_OK;
+}

@@ -51,6 +51,7 @@ struct FeatParams {
   int32_t n_feat;            // G + nb * n_channels
   int32_t n_blocks, n_pairs, k_splits;
   double* gram;              // [n_cg, n_feat, n_feat] (+=), upper block triangle
+  const double* frame_w;     // [n_frames] frame weights, frame-aligned with forces (weighted Grams only)
 };
 
 template <typename T>
@@ -84,7 +85,8 @@ __device__ __forceinline__ void clipped_gauss(double d, double mu, double inv_w,
 }
 
 // Fills panel rows (t,d) x 128 feature columns [col0, col0+128) for the chunk [t0, t0+nf).
-template <typename T>
+// W: the rows of frame t are multiplied by sqrt(frame_w[t]) once complete (weighted fits).
+template <typename T, bool W>
 __device__ __forceinline__ void fill_feat_panel(const FeatParams& p, const T* __restrict__ coords,
                                                 const T* __restrict__ forces, int64_t t0, int nf, int col0,
                                                 const double (*__restrict__ bead_pos)[3], double* __restrict__ panel) {
@@ -112,10 +114,17 @@ __device__ __forceinline__ void fill_feat_panel(const FeatParams& p, const T* __
     const int t = item / per_frame, u = item - t * per_frame;
     const T* fr_f = forces + (t0 + t) * fstride;
     double* row = panel + (t * 3) * kFgStride;
+    double sw = 1.0;
+    if constexpr (W) sw = sqrt(__ldg(p.frame_w + t0 + t));
     if (u < n_id) {
       const int g = id_lo + u;
       double f[3], m;
       group_sum<T>(fr_f, p.grp_ptr, p.grp_sites, g, f, m);
+      if constexpr (W) {
+        f[0] *= sw;
+        f[1] *= sw;
+        f[2] *= sw;
+      }
       const int x = g - col0;
       row[x] = f[0];
       row[kFgStride + x] = f[1];
@@ -138,9 +147,15 @@ __device__ __forceinline__ void fill_feat_panel(const FeatParams& p, const T* __
         clipped_gauss(dist, __ldg(p.centers + k), p.inv_width, p.clip, p.ln_inv_clip, g, gp);
         const double c = p.kbt * m * gp;
         const int x = col - col0;
-        row[x] = g * f[0] + c * ux;
-        row[kFgStride + x] = g * f[1] + c * uy;
-        row[2 * kFgStride + x] = g * f[2] + c * uz;
+        double v0 = g * f[0] + c * ux, v1 = g * f[1] + c * uy, v2 = g * f[2] + c * uz;
+        if constexpr (W) {
+          v0 *= sw;
+          v1 *= sw;
+          v2 *= sw;
+        }
+        row[x] = v0;
+        row[kFgStride + x] = v1;
+        row[2 * kFgStride + x] = v2;
       }
     }
   }
@@ -162,7 +177,7 @@ __device__ __forceinline__ void bead_positions(const FeatParams& p, const T* __r
   }
 }
 
-template <typename T>
+template <typename T, bool W>
 __global__ void __launch_bounds__(kFgThreads, 1) feat_gram_kernel(const __grid_constant__ FeatParams p) {
   constexpr int KROWS = 3 * kFgKF;
   extern __shared__ __align__(128) unsigned char smem[];
@@ -202,8 +217,8 @@ __global__ void __launch_bounds__(kFgThreads, 1) feat_gram_kernel(const __grid_c
     const int nf = (int)min((int64_t)kFgKF, p.n_frames - t0);
     bead_positions<T>(p, coords, t0, nf, bead, bead_pos);
     __syncthreads();
-    fill_feat_panel<T>(p, coords, forces, t0, nf, bi * kFgBlock, bead_pos, panel_i);
-    if (!diag) fill_feat_panel<T>(p, coords, forces, t0, nf, bj * kFgBlock, bead_pos, panel_j);
+    fill_feat_panel<T, W>(p, coords, forces, t0, nf, bi * kFgBlock, bead_pos, panel_i);
+    if (!diag) fill_feat_panel<T, W>(p, coords, forces, t0, nf, bj * kFgBlock, bead_pos, panel_j);
     __syncthreads();
 #pragma unroll 2
     for (int kk = 0; kk < KROWS / 4; ++kk) {
@@ -242,7 +257,7 @@ __global__ void __launch_bounds__(kFgThreads, 1) feat_gram_kernel(const __grid_c
 // Phase 1 (thread per (frame, group)): group force, distance to the bead and unit vector into
 // shared memory.  Phase 2 (thread per (frame, feature column)): one clipped Gaussian each, stores
 // of consecutive threads fall on consecutive addresses of a panel row.
-template <typename T>
+template <typename T, bool W>
 __global__ void __launch_bounds__(256) feat_pack_kernel(const __grid_constant__ FeatParams p, double* __restrict__ ws) {
   extern __shared__ __align__(16) unsigned char fp_smem[];
   __shared__ double bead_pos[kPanelKF][3];
@@ -306,6 +321,12 @@ __global__ void __launch_bounds__(256) feat_pack_kernel(const __grid_constant__ 
       v0 = gk * rec[0] + c * rec[4];
       v1 = gk * rec[1] + c * rec[5];
       v2 = gk * rec[2] + c * rec[6];
+    }
+    if constexpr (W) {
+      const double sw = sqrt(__ldg(p.frame_w + t0 + t));
+      v0 *= sw;
+      v1 *= sw;
+      v2 *= sw;
     }
     double* dst = slab + (int64_t)(col >> 7) * kPanelElems + (t * 3) * kPanelStride + (col & 127);
     dst[0] = v0;
@@ -751,12 +772,21 @@ static int fill_params(FeatParams& p, const void* coords, const void* forces, in
 
 }  // namespace agf
 
-extern "C" int agf_gram_feat(const void* coords, const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
-                             const int32_t* grp_ptr, const int32_t* grp_sites, int32_t n_groups,
-                             int32_t n_channels, const int32_t* bead_ptr, const int32_t* bead_sites,
-                             const double* bead_w, int32_t n_cg, const double* centers, int32_t nb, double width,
-                             double clip, double kbt, double* gram, void* stream) {
-  using namespace agf;
+namespace agf {
+
+template <typename T, bool W>
+static int launch_feat_gram(const FeatParams& p, int grid, size_t smem, cudaStream_t s) {
+  AGF_CUDA_TRY(cudaFuncSetAttribute(feat_gram_kernel<T, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  feat_gram_kernel<T, W><<<grid, kFgThreads, smem, s>>>(p);
+  return AGF_OK;
+}
+
+// Both public forms of each Gram share one host path: frame_weights == NULL is the unweighted Gram.
+static int gram_feat_impl(const void* coords, const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                          const int32_t* grp_ptr, const int32_t* grp_sites, int32_t n_groups, int32_t n_channels,
+                          const int32_t* bead_ptr, const int32_t* bead_sites, const double* bead_w, int32_t n_cg,
+                          const double* centers, int32_t nb, double width, double clip, double kbt, double* gram,
+                          const double* frame_weights, void* stream) {
   FeatParams p;
   int rc = fill_params(p, coords, forces, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels, bead_ptr,
                        bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt);
@@ -765,6 +795,7 @@ extern "C" int agf_gram_feat(const void* coords, const void* forces, int dtype, 
   AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_gram_feat: bad dtype");
   if (n_frames == 0) return AGF_OK;
   p.gram = gram;
+  p.frame_w = frame_weights;
   const int64_t n_chunks = (n_frames + kFgKF - 1) / kFgKF;
   int64_t items = (int64_t)n_cg * p.n_pairs;
   int64_t ks = (2LL * sm_count() + items - 1) / items;
@@ -774,15 +805,93 @@ extern "C" int agf_gram_feat(const void* coords, const void* forces, int dtype, 
   const size_t smem = (size_t)2 * 3 * kFgKF * kFgStride * sizeof(double);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const int grid = (int)(items * ks);
-  if (dtype == AGF_F32) {
-    AGF_CUDA_TRY(cudaFuncSetAttribute(feat_gram_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    feat_gram_kernel<float><<<grid, kFgThreads, smem, s>>>(p);
-  } else {
-    AGF_CUDA_TRY(cudaFuncSetAttribute(feat_gram_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    feat_gram_kernel<double><<<grid, kFgThreads, smem, s>>>(p);
-  }
+  if (dtype == AGF_F32)
+    rc = frame_weights ? launch_feat_gram<float, true>(p, grid, smem, s) : launch_feat_gram<float, false>(p, grid, smem, s);
+  else
+    rc = frame_weights ? launch_feat_gram<double, true>(p, grid, smem, s)
+                       : launch_feat_gram<double, false>(p, grid, smem, s);
+  if (rc) return rc;
   AGF_CUDA_TRY(cudaGetLastError());
   return AGF_OK;
+}
+
+template <typename T, bool W>
+static int launch_feat_pack(const FeatParams& p, int64_t grid, size_t smem, double* ws, cudaStream_t s) {
+  AGF_CUDA_TRY(cudaFuncSetAttribute(feat_pack_kernel<T, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  feat_pack_kernel<T, W><<<(unsigned)grid, 256, smem, s>>>(p, ws);
+  return AGF_OK;
+}
+
+static int gram_feat_ws_impl(const void* coords, const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                             const int32_t* grp_ptr, const int32_t* grp_sites, int32_t n_groups, int32_t n_channels,
+                             const int32_t* bead_ptr, const int32_t* bead_sites, const double* bead_w, int32_t n_cg,
+                             const double* centers, int32_t nb, double width, double clip, double kbt, double* gram,
+                             void* workspace, size_t workspace_bytes, const double* frame_weights, void* stream) {
+  FeatParams p;
+  int rc = fill_params(p, coords, forces, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels, bead_ptr,
+                       bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt);
+  if (rc) return rc;
+  AGF_REQUIRE(forces && gram, "agf_gram_feat_ws: null pointer");
+  AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_gram_feat_ws: bad dtype");
+  const int64_t per_chunk = (int64_t)n_cg * p.n_blocks * kPanelBytes;
+  const size_t pack_smem = (size_t)kPanelKF * n_groups * 8 * sizeof(double);
+  if (workspace == nullptr || (int64_t)workspace_bytes < per_chunk)
+    return gram_feat_impl(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels, bead_ptr,
+                          bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, frame_weights, stream);
+  AGF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) % 16) == 0, "agf_gram_feat_ws: workspace must be 16-byte aligned");
+  if (n_frames == 0) return AGF_OK;
+  if (pack_smem > (size_t)200 * 1024)  // > 3200 constraint groups: per-frame records do not fit in shared memory
+    return gram_feat_impl(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels, bead_ptr,
+                          bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, frame_weights, stream);
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const int64_t slab_chunks = (int64_t)workspace_bytes / per_chunk;
+  const int64_t slab_frames = slab_chunks * kPanelKF;
+  const size_t elem = dtype == AGF_F32 ? 4 : 8;
+  const size_t frame_bytes = (size_t)n_sites * 3 * elem;
+  for (int64_t f0 = 0; f0 < n_frames; f0 += slab_frames) {
+    const int64_t nf = n_frames - f0 < slab_frames ? n_frames - f0 : slab_frames;
+    const int64_t chunks = (nf + kPanelKF - 1) / kPanelKF;
+    p.coords = reinterpret_cast<const char*>(coords) + (size_t)f0 * frame_bytes;
+    p.forces = reinterpret_cast<const char*>(forces) + (size_t)f0 * frame_bytes;
+    p.frame_w = frame_weights ? frame_weights + f0 : nullptr;
+    p.n_frames = nf;
+    const int64_t grid = chunks * n_cg;
+    AGF_REQUIRE(grid < (int64_t)1 << 31, "agf_gram_feat_ws: slab too large");
+    double* ws = reinterpret_cast<double*>(workspace);
+    if (dtype == AGF_F32)
+      rc = frame_weights ? launch_feat_pack<float, true>(p, grid, pack_smem, ws, s)
+                         : launch_feat_pack<float, false>(p, grid, pack_smem, ws, s);
+    else
+      rc = frame_weights ? launch_feat_pack<double, true>(p, grid, pack_smem, ws, s)
+                         : launch_feat_pack<double, false>(p, grid, pack_smem, ws, s);
+    if (rc) return rc;
+    AGF_CUDA_TRY(cudaGetLastError());
+    rc = launch_panel_syrk(reinterpret_cast<const double*>(workspace), chunks, p.n_feat, n_cg, gram, s);
+    if (rc) return rc;
+  }
+  return AGF_OK;
+}
+
+}  // namespace agf
+
+extern "C" int agf_gram_feat(const void* coords, const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                             const int32_t* grp_ptr, const int32_t* grp_sites, int32_t n_groups,
+                             int32_t n_channels, const int32_t* bead_ptr, const int32_t* bead_sites,
+                             const double* bead_w, int32_t n_cg, const double* centers, int32_t nb, double width,
+                             double clip, double kbt, double* gram, void* stream) {
+  return agf::gram_feat_impl(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels,
+                             bead_ptr, bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, nullptr, stream);
+}
+
+extern "C" int agf_gram_feat_weighted(const void* coords, const void* forces, int dtype, int64_t n_frames,
+                                      int32_t n_sites, const int32_t* grp_ptr, const int32_t* grp_sites,
+                                      int32_t n_groups, int32_t n_channels, const int32_t* bead_ptr,
+                                      const int32_t* bead_sites, const double* bead_w, int32_t n_cg,
+                                      const double* centers, int32_t nb, double width, double clip, double kbt,
+                                      double* gram, const double* frame_weights, void* stream) {
+  return agf::gram_feat_impl(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels,
+                             bead_ptr, bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, frame_weights,
+                             stream);
 }
 
 extern "C" size_t agf_gram_feat_workspace_bytes(int32_t n_groups, int32_t n_channels, int32_t nb, int32_t n_cg,
@@ -805,47 +914,21 @@ extern "C" int agf_gram_feat_ws(const void* coords, const void* forces, int dtyp
                                 const double* bead_w, int32_t n_cg, const double* centers, int32_t nb, double width,
                                 double clip, double kbt, double* gram, void* workspace, size_t workspace_bytes,
                                 void* stream) {
-  using namespace agf;
-  FeatParams p;
-  int rc = fill_params(p, coords, forces, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels, bead_ptr,
-                       bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt);
-  if (rc) return rc;
-  AGF_REQUIRE(forces && gram, "agf_gram_feat_ws: null pointer");
-  AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_gram_feat_ws: bad dtype");
-  const int64_t per_chunk = (int64_t)n_cg * p.n_blocks * kPanelBytes;
-  if (workspace == nullptr || (int64_t)workspace_bytes < per_chunk)
-    return agf_gram_feat(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels, bead_ptr,
-                         bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, stream);
-  AGF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) % 16) == 0, "agf_gram_feat_ws: workspace must be 16-byte aligned");
-  if (n_frames == 0) return AGF_OK;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const int64_t slab_chunks = (int64_t)workspace_bytes / per_chunk;
-  const int64_t slab_frames = slab_chunks * kPanelKF;
-  const size_t elem = dtype == AGF_F32 ? 4 : 8;
-  const size_t frame_bytes = (size_t)n_sites * 3 * elem;
-  const size_t pack_smem = (size_t)kPanelKF * n_groups * 8 * sizeof(double);
-  if (pack_smem > (size_t)200 * 1024)  // > 3200 constraint groups: per-frame records do not fit in shared memory
-    return agf_gram_feat(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels, bead_ptr,
-                         bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, stream);
-  AGF_CUDA_TRY(cudaFuncSetAttribute(feat_pack_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pack_smem));
-  AGF_CUDA_TRY(cudaFuncSetAttribute(feat_pack_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pack_smem));
-  for (int64_t f0 = 0; f0 < n_frames; f0 += slab_frames) {
-    const int64_t nf = n_frames - f0 < slab_frames ? n_frames - f0 : slab_frames;
-    const int64_t chunks = (nf + kPanelKF - 1) / kPanelKF;
-    p.coords = reinterpret_cast<const char*>(coords) + (size_t)f0 * frame_bytes;
-    p.forces = reinterpret_cast<const char*>(forces) + (size_t)f0 * frame_bytes;
-    p.n_frames = nf;
-    const int64_t grid = chunks * n_cg;
-    AGF_REQUIRE(grid < (int64_t)1 << 31, "agf_gram_feat_ws: slab too large");
-    if (dtype == AGF_F32)
-      feat_pack_kernel<float><<<(unsigned)grid, 256, pack_smem, s>>>(p, reinterpret_cast<double*>(workspace));
-    else
-      feat_pack_kernel<double><<<(unsigned)grid, 256, pack_smem, s>>>(p, reinterpret_cast<double*>(workspace));
-    AGF_CUDA_TRY(cudaGetLastError());
-    rc = launch_panel_syrk(reinterpret_cast<const double*>(workspace), chunks, p.n_feat, n_cg, gram, s);
-    if (rc) return rc;
-  }
-  return AGF_OK;
+  return agf::gram_feat_ws_impl(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels,
+                                bead_ptr, bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, workspace,
+                                workspace_bytes, nullptr, stream);
+}
+
+extern "C" int agf_gram_feat_ws_weighted(const void* coords, const void* forces, int dtype, int64_t n_frames,
+                                         int32_t n_sites, const int32_t* grp_ptr, const int32_t* grp_sites,
+                                         int32_t n_groups, int32_t n_channels, const int32_t* bead_ptr,
+                                         const int32_t* bead_sites, const double* bead_w, int32_t n_cg,
+                                         const double* centers, int32_t nb, double width, double clip, double kbt,
+                                         double* gram, void* workspace, size_t workspace_bytes,
+                                         const double* frame_weights, void* stream) {
+  return agf::gram_feat_ws_impl(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels,
+                                bead_ptr, bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, workspace,
+                                workspace_bytes, frame_weights, stream);
 }
 
 extern "C" size_t agf_gram_feat_i8_workspace_bytes(int32_t n_groups, int32_t n_channels, int32_t nb, int32_t n_cg,

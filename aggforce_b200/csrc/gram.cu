@@ -58,6 +58,7 @@ struct GramParams {
   int32_t n_pairs;   // n_blocks (n_blocks + 1) / 2
   int32_t k_splits;  // CTAs per block pair
   double* gram;
+  const double* weights;  // [n_frames] frame weights (read by the weighted instantiations only)
   ChunkSchedule sch;
 };
 
@@ -156,14 +157,18 @@ __device__ __forceinline__ void tri_store(const double (&acc)[kMaxTriSlots][2], 
 }
 
 // ------------------------------------------------------------------ panel fill (group sum + f64 promotion)
-template <typename T, bool GLOBAL>
+// W: the group sums of frame t are scaled by sqrt(weights[t]) (weighted fits; see agf_gram_linear_weighted).
+template <typename T, bool GLOBAL, bool W>
 __device__ __forceinline__ void fill_panel(const T* __restrict__ frames, int nf, int kf, int n_sites,
                                            const int32_t* __restrict__ col_ptr,
                                            const int32_t* __restrict__ col_sites, int col0, int n_red,
-                                           int width_pad, double* __restrict__ panel) {
+                                           int width_pad, const double* __restrict__ weights,
+                                           double* __restrict__ panel) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int t = warp; t < kf; t += kGramWarps) {
     const T* fr = frames + (int64_t)t * n_sites * 3;
+    double sw = 1.0;
+    if constexpr (W) sw = t < nf ? sqrt(__ldg(weights + t)) : 0.0;
     for (int x = lane; x < width_pad; x += 32) {
       double s0 = 0.0, s1 = 0.0, s2 = 0.0;
       const int col = col0 + x;
@@ -181,6 +186,11 @@ __device__ __forceinline__ void fill_panel(const T* __restrict__ frames, int nf,
             s2 += to_f64(p[2]);
           }
         }
+      }
+      if constexpr (W) {
+        s0 *= sw;
+        s1 *= sw;
+        s2 *= sw;
       }
       double* dst = panel + (t * 3) * kStride + x;
       dst[0] = s0;
@@ -222,7 +232,7 @@ constexpr int kTriThreads = (kMmaWarps + kFillWarps) * 32;
 constexpr int kFillThreads = kFillWarps * 32;
 constexpr int kRawStages = 3;
 
-template <typename T, int KF, int NT>
+template <typename T, int KF, int NT, bool W>
 __global__ void __launch_bounds__(kTriThreads, 1) gram_tri_kernel(const __grid_constant__ GramParams p) {
   constexpr int KROWS = 3 * KF;
   constexpr int NCOLS = NT * 8;
@@ -340,11 +350,14 @@ __global__ void __launch_bounds__(kTriThreads, 1) gram_tri_kernel(const __grid_c
       mbar_wait(&panel_empty[pb], (uint32_t)(((j >> 1) & 1) ^ 1));
       double* panel = panel0 + (size_t)pb * KROWS * kStride;
       const uint32_t raw_u32 = smem_u32(stage_ptr), panel_u32 = smem_u32(panel);
+      const double* chunk_w = W ? p.weights + p.sch.start(c) : nullptr;
       if (!generic) {
         for (int t = fw; t < KF; t += kFillWarps) {
           const uint32_t rbase = raw_u32 + (uint32_t)t * frame_bytes;
           const uint32_t pbase = panel_u32 + (uint32_t)(t * 3 * kStride * 8);
           const bool live = t < nf;
+          double sw = 1.0;  // one multiply per value where the group sum is complete (DMUL, like DADD, shares the DMMA pipe)
+          if constexpr (W) sw = live ? sqrt(__ldg(chunk_w + t)) : 0.0;
 #pragma unroll
           for (int gi = 0; gi < NG; ++gi) {
             double s0 = 0.0, s1 = 0.0, s2 = 0.0;
@@ -371,6 +384,11 @@ __global__ void __launch_bounds__(kTriThreads, 1) gram_tri_kernel(const __grid_c
                 }
               }
             }
+            if constexpr (W) {
+              s0 *= sw;
+              s1 *= sw;
+              s2 *= sw;
+            }
             if (gi * 32 + lane < p.n_red) {
               const uint32_t d = pbase + coff[gi];
               sts_f64(d, s0);
@@ -390,6 +408,12 @@ __global__ void __launch_bounds__(kTriThreads, 1) gram_tri_kernel(const __grid_c
               s0 += to_f64(q[0]);
               s1 += to_f64(q[1]);
               s2 += to_f64(q[2]);
+            }
+            if constexpr (W) {
+              const double sw = sqrt(__ldg(chunk_w + t));
+              s0 *= sw;
+              s1 *= sw;
+              s2 *= sw;
             }
           }
           double* dst = panel + (t * 3) * kStride + x;
@@ -442,7 +466,7 @@ __global__ void __launch_bounds__(kTriThreads, 1) gram_tri_kernel(const __grid_c
 
 // ------------------------------------------------------------------ block pairs (any n_red), global gather
 // CTA = block pair (I <= J) x k-split; warp w owns tile rows {2w, 2w+1} x all 16 tile columns.
-template <typename T, int KF>
+template <typename T, int KF, bool W>
 __global__ void __launch_bounds__(kGramThreads, 1) gram_block_kernel(const __grid_constant__ GramParams p) {
   constexpr int KROWS = 3 * KF;
   extern __shared__ __align__(128) unsigned char smem[];
@@ -478,9 +502,11 @@ __global__ void __launch_bounds__(kGramThreads, 1) gram_block_kernel(const __gri
     const int nf = p.sch.count(c);
     if (nf > 0) {
       const T* src = forces + p.sch.start(c) * (int64_t)p.n_sites * 3;
-      fill_panel<T, true>(src, nf, KF, p.n_sites, p.col_ptr, p.col_sites, col0_i, p.n_red, kBlockCols, panel_i);
+      const double* w = W ? p.weights + p.sch.start(c) : nullptr;
+      fill_panel<T, true, W>(src, nf, KF, p.n_sites, p.col_ptr, p.col_sites, col0_i, p.n_red, kBlockCols, w, panel_i);
       if (!diag)
-        fill_panel<T, true>(src, nf, KF, p.n_sites, p.col_ptr, p.col_sites, col0_j, p.n_red, kBlockCols, panel_j);
+        fill_panel<T, true, W>(src, nf, KF, p.n_sites, p.col_ptr, p.col_sites, col0_j, p.n_red, kBlockCols, w,
+                               panel_j);
     }
     __syncthreads();
     if (nf > 0) {
@@ -526,11 +552,12 @@ constexpr int kWsKF = kPanelKF;
 constexpr int kWsPanel = kPanelElems;  // doubles per (chunk, block)
 static_assert(kStride == kPanelStride && kBlockCols == kPanelCols, "panel geometry");
 
-template <typename T>
+template <typename T, bool W>
 __global__ void __launch_bounds__(256) gram_pack_kernel(const T* __restrict__ forces, int64_t n_frames, int n_sites,
                                                         const int32_t* __restrict__ col_ptr,
                                                         const int32_t* __restrict__ col_sites, int n_red,
-                                                        int n_blocks, double* __restrict__ ws) {
+                                                        int n_blocks, const double* __restrict__ weights,
+                                                        double* __restrict__ ws) {
   const int64_t chunk = blockIdx.x / n_blocks;
   const int blk = blockIdx.x - (int)(chunk * n_blocks);
   const int64_t t0 = chunk * kWsKF;
@@ -548,6 +575,12 @@ __global__ void __launch_bounds__(256) gram_pack_kernel(const T* __restrict__ fo
         s0 += to_f64(__ldg(p));
         s1 += to_f64(__ldg(p + 1));
         s2 += to_f64(__ldg(p + 2));
+      }
+      if constexpr (W) {
+        const double sw = sqrt(__ldg(weights + t0 + t));
+        s0 *= sw;
+        s1 *= sw;
+        s2 *= sw;
       }
     }
     double* dst = panel + (t * 3) * kStride + x;
@@ -658,9 +691,9 @@ __global__ void symmetrize_kernel(double* g, int n) {
   if (i > j) g[idx] = g[(int64_t)j * n + i];
 }
 
-template <typename T, int KF, int NT>
+template <typename T, int KF, int NT, bool W>
 static int launch_tri(GramParams& p, size_t smem, int ctas, cudaStream_t stream) {
-  auto kern = gram_tri_kernel<T, KF, NT>;
+  auto kern = gram_tri_kernel<T, KF, NT, W>;
   AGF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<ctas, kTriThreads, smem, stream>>>(p);
   AGF_CUDA_TRY(cudaGetLastError());
@@ -675,7 +708,7 @@ static size_t tri_smem_bytes(const GramParams& p) {
   return off + kRawStages * stage_bytes;
 }
 
-template <typename T, int KF>
+template <typename T, int KF, bool W>
 static int dispatch_tri(GramParams& p, cudaStream_t stream) {
   const int sms = sm_count();
   p.sch = make_schedule(p.forces, p.n_frames, (int64_t)p.n_sites * 3 * sizeof(T), KF);
@@ -683,33 +716,33 @@ static int dispatch_tri(GramParams& p, cudaStream_t stream) {
   int64_t want = p.sch.n_chunks;
   int ctas = (int)(want < sms ? (want < 1 ? 1 : want) : sms);
   switch ((p.n_red + 7) / 8) {
-    case 1: return launch_tri<T, KF, 1>(p, smem, ctas, stream);
-    case 2: return launch_tri<T, KF, 2>(p, smem, ctas, stream);
-    case 3: return launch_tri<T, KF, 3>(p, smem, ctas, stream);
-    case 4: return launch_tri<T, KF, 4>(p, smem, ctas, stream);
-    case 5: return launch_tri<T, KF, 5>(p, smem, ctas, stream);
-    case 6: return launch_tri<T, KF, 6>(p, smem, ctas, stream);
-    case 7: return launch_tri<T, KF, 7>(p, smem, ctas, stream);
-    case 8: return launch_tri<T, KF, 8>(p, smem, ctas, stream);
-    case 9: return launch_tri<T, KF, 9>(p, smem, ctas, stream);
-    case 10: return launch_tri<T, KF, 10>(p, smem, ctas, stream);
-    case 11: return launch_tri<T, KF, 11>(p, smem, ctas, stream);
-    case 12: return launch_tri<T, KF, 12>(p, smem, ctas, stream);
-    case 13: return launch_tri<T, KF, 13>(p, smem, ctas, stream);
-    case 14: return launch_tri<T, KF, 14>(p, smem, ctas, stream);
-    case 15: return launch_tri<T, KF, 15>(p, smem, ctas, stream);
-    default: return launch_tri<T, KF, 16>(p, smem, ctas, stream);
+    case 1: return launch_tri<T, KF, 1, W>(p, smem, ctas, stream);
+    case 2: return launch_tri<T, KF, 2, W>(p, smem, ctas, stream);
+    case 3: return launch_tri<T, KF, 3, W>(p, smem, ctas, stream);
+    case 4: return launch_tri<T, KF, 4, W>(p, smem, ctas, stream);
+    case 5: return launch_tri<T, KF, 5, W>(p, smem, ctas, stream);
+    case 6: return launch_tri<T, KF, 6, W>(p, smem, ctas, stream);
+    case 7: return launch_tri<T, KF, 7, W>(p, smem, ctas, stream);
+    case 8: return launch_tri<T, KF, 8, W>(p, smem, ctas, stream);
+    case 9: return launch_tri<T, KF, 9, W>(p, smem, ctas, stream);
+    case 10: return launch_tri<T, KF, 10, W>(p, smem, ctas, stream);
+    case 11: return launch_tri<T, KF, 11, W>(p, smem, ctas, stream);
+    case 12: return launch_tri<T, KF, 12, W>(p, smem, ctas, stream);
+    case 13: return launch_tri<T, KF, 13, W>(p, smem, ctas, stream);
+    case 14: return launch_tri<T, KF, 14, W>(p, smem, ctas, stream);
+    case 15: return launch_tri<T, KF, 15, W>(p, smem, ctas, stream);
+    default: return launch_tri<T, KF, 16, W>(p, smem, ctas, stream);
   }
 }
 
 // KFBIG / KFSMALL: frames per chunk of the staged kernel (the larger one when it fits in smem).
-template <typename T, int KFBIG, int KFSMALL>
+template <typename T, int KFBIG, int KFSMALL, bool W>
 static int launch_gram(GramParams& p, cudaStream_t stream) {
   const int sms = sm_count();
   const size_t budget = 226 * 1024;
   if (p.n_blocks == 1) {
-    if (tri_smem_bytes<T, KFBIG>(p) <= budget) return dispatch_tri<T, KFBIG>(p, stream);
-    if (tri_smem_bytes<T, KFSMALL>(p) <= budget) return dispatch_tri<T, KFSMALL>(p, stream);
+    if (tri_smem_bytes<T, KFBIG>(p) <= budget) return dispatch_tri<T, KFBIG, W>(p, stream);
+    if (tri_smem_bytes<T, KFSMALL>(p) <= budget) return dispatch_tri<T, KFSMALL, W>(p, stream);
     // frames too wide to stage in shared memory: use the gather variant
   }
   constexpr int KF = KFSMALL;
@@ -719,19 +752,16 @@ static int launch_gram(GramParams& p, cudaStream_t stream) {
   if (ks > p.sch.n_chunks) ks = p.sch.n_chunks;
   if (ks < 1) ks = 1;
   p.k_splits = (int32_t)ks;
-  auto kern = gram_block_kernel<T, KF>;
+  auto kern = gram_block_kernel<T, KF, W>;
   AGF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<p.k_splits * p.n_pairs, kGramThreads, smem, stream>>>(p);
   AGF_CUDA_TRY(cudaGetLastError());
   return AGF_OK;
 }
 
-}  // namespace agf
-
-extern "C" int agf_gram_linear(const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
-                               const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red, double* gram,
-                               void* stream) {
-  using namespace agf;
+static int gram_linear_impl(const void* forces, int dtype, int64_t n_frames, int32_t n_sites, const int32_t* col_ptr,
+                            const int32_t* col_sites, int32_t n_red, double* gram, const double* weights,
+                            void* stream) {
   AGF_REQUIRE(forces && col_ptr && col_sites && gram, "agf_gram_linear: null pointer");
   AGF_REQUIRE(n_frames >= 0 && n_sites > 0 && n_red > 0, "agf_gram_linear: bad sizes T=%lld n=%d n_red=%d",
               (long long)n_frames, n_sites, n_red);
@@ -746,11 +776,78 @@ extern "C" int agf_gram_linear(const void* forces, int dtype, int64_t n_frames, 
   p.col_sites = col_sites;
   p.n_red = n_red;
   p.gram = gram;
+  p.weights = weights;
   p.n_blocks = (n_red + kBlockCols - 1) / kBlockCols;
   p.n_pairs = p.n_blocks * (p.n_blocks + 1) / 2;
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  if (dtype == AGF_F32) return launch_gram<float, 16, 8>(p, s);
-  return launch_gram<double, 8, 4>(p, s);
+  if (weights) {
+    if (dtype == AGF_F32) return launch_gram<float, 16, 8, true>(p, s);
+    return launch_gram<double, 8, 4, true>(p, s);
+  }
+  if (dtype == AGF_F32) return launch_gram<float, 16, 8, false>(p, s);
+  return launch_gram<double, 8, 4, false>(p, s);
+}
+
+template <typename T>
+static void launch_pack(const T* forces, int64_t nf, int32_t n_sites, const int32_t* col_ptr, const int32_t* col_sites,
+                        int32_t n_red, int n_blocks, const double* weights, double* ws, int64_t grid, cudaStream_t s) {
+  if (weights)
+    gram_pack_kernel<T, true><<<(unsigned)grid, 256, 0, s>>>(forces, nf, n_sites, col_ptr, col_sites, n_red, n_blocks,
+                                                             weights, ws);
+  else
+    gram_pack_kernel<T, false><<<(unsigned)grid, 256, 0, s>>>(forces, nf, n_sites, col_ptr, col_sites, n_red, n_blocks,
+                                                              nullptr, ws);
+}
+
+static int gram_linear_ws_impl(const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                               const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red, double* gram,
+                               void* workspace, size_t workspace_bytes, const double* weights, void* stream) {
+  AGF_REQUIRE(forces && col_ptr && col_sites && gram, "agf_gram_linear_ws: null pointer");
+  AGF_REQUIRE(n_frames >= 0 && n_sites > 0 && n_red > 0, "agf_gram_linear_ws: bad sizes");
+  AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_gram_linear_ws: bad dtype");
+  const int64_t n_blocks = (n_red + kBlockCols - 1) / kBlockCols;
+  const int64_t per_chunk = n_blocks * kWsPanel * (int64_t)sizeof(double);
+  if (n_red <= kBlockCols || workspace == nullptr || (int64_t)workspace_bytes < per_chunk)
+    return gram_linear_impl(forces, dtype, n_frames, n_sites, col_ptr, col_sites, n_red, gram, weights, stream);
+  AGF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) % 16) == 0, "agf_gram_linear_ws: workspace must be 16-byte aligned");
+  if (n_frames == 0) return AGF_OK;
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const int64_t slab_chunks = (int64_t)workspace_bytes / per_chunk;
+  const int64_t slab_frames = slab_chunks * kWsKF;
+  const size_t elem = dtype == AGF_F32 ? 4 : 8;
+  for (int64_t f0 = 0; f0 < n_frames; f0 += slab_frames) {
+    const int64_t nf = n_frames - f0 < slab_frames ? n_frames - f0 : slab_frames;
+    const int64_t chunks = (nf + kWsKF - 1) / kWsKF;
+    const char* src = reinterpret_cast<const char*>(forces) + (size_t)f0 * n_sites * 3 * elem;
+    const double* w = weights ? weights + f0 : nullptr;
+    const int64_t pack_grid = chunks * n_blocks;
+    AGF_REQUIRE(pack_grid < (int64_t)1 << 31, "agf_gram_linear_ws: slab too large");
+    if (dtype == AGF_F32)
+      launch_pack(reinterpret_cast<const float*>(src), nf, n_sites, col_ptr, col_sites, n_red, (int)n_blocks, w,
+                  reinterpret_cast<double*>(workspace), pack_grid, s);
+    else
+      launch_pack(reinterpret_cast<const double*>(src), nf, n_sites, col_ptr, col_sites, n_red, (int)n_blocks, w,
+                  reinterpret_cast<double*>(workspace), pack_grid, s);
+    AGF_CUDA_TRY(cudaGetLastError());
+    int rc = launch_panel_syrk(reinterpret_cast<const double*>(workspace), chunks, n_red, 1, gram, s);
+    if (rc) return rc;
+  }
+  return AGF_OK;
+}
+
+}  // namespace agf
+
+extern "C" int agf_gram_linear(const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                               const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red, double* gram,
+                               void* stream) {
+  return agf::gram_linear_impl(forces, dtype, n_frames, n_sites, col_ptr, col_sites, n_red, gram, nullptr, stream);
+}
+
+extern "C" int agf_gram_linear_weighted(const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                                        const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red, double* gram,
+                                        const double* frame_weights, void* stream) {
+  return agf::gram_linear_impl(forces, dtype, n_frames, n_sites, col_ptr, col_sites, n_red, gram, frame_weights,
+                               stream);
 }
 
 extern "C" size_t agf_gram_linear_workspace_bytes(int32_t n_sites, int32_t n_red, int64_t n_frames) {
@@ -770,39 +867,16 @@ extern "C" size_t agf_gram_linear_workspace_bytes(int32_t n_sites, int32_t n_red
 extern "C" int agf_gram_linear_ws(const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
                                   const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red, double* gram,
                                   void* workspace, size_t workspace_bytes, void* stream) {
-  using namespace agf;
-  AGF_REQUIRE(forces && col_ptr && col_sites && gram, "agf_gram_linear_ws: null pointer");
-  AGF_REQUIRE(n_frames >= 0 && n_sites > 0 && n_red > 0, "agf_gram_linear_ws: bad sizes");
-  AGF_REQUIRE(dtype == AGF_F32 || dtype == AGF_F64, "agf_gram_linear_ws: bad dtype");
-  const int64_t n_blocks = (n_red + kBlockCols - 1) / kBlockCols;
-  const int64_t per_chunk = n_blocks * kWsPanel * (int64_t)sizeof(double);
-  if (n_red <= kBlockCols || workspace == nullptr || (int64_t)workspace_bytes < per_chunk)
-    return agf_gram_linear(forces, dtype, n_frames, n_sites, col_ptr, col_sites, n_red, gram, stream);
-  AGF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) % 16) == 0, "agf_gram_linear_ws: workspace must be 16-byte aligned");
-  if (n_frames == 0) return AGF_OK;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const int64_t slab_chunks = (int64_t)workspace_bytes / per_chunk;
-  const int64_t slab_frames = slab_chunks * kWsKF;
-  const size_t elem = dtype == AGF_F32 ? 4 : 8;
-  for (int64_t f0 = 0; f0 < n_frames; f0 += slab_frames) {
-    const int64_t nf = n_frames - f0 < slab_frames ? n_frames - f0 : slab_frames;
-    const int64_t chunks = (nf + kWsKF - 1) / kWsKF;
-    const char* src = reinterpret_cast<const char*>(forces) + (size_t)f0 * n_sites * 3 * elem;
-    const int64_t pack_grid = chunks * n_blocks;
-    AGF_REQUIRE(pack_grid < (int64_t)1 << 31, "agf_gram_linear_ws: slab too large");
-    if (dtype == AGF_F32)
-      gram_pack_kernel<float><<<(unsigned)pack_grid, 256, 0, s>>>(reinterpret_cast<const float*>(src), nf, n_sites,
-                                                                  col_ptr, col_sites, n_red, (int)n_blocks,
-                                                                  reinterpret_cast<double*>(workspace));
-    else
-      gram_pack_kernel<double><<<(unsigned)pack_grid, 256, 0, s>>>(reinterpret_cast<const double*>(src), nf, n_sites,
-                                                                   col_ptr, col_sites, n_red, (int)n_blocks,
-                                                                   reinterpret_cast<double*>(workspace));
-    AGF_CUDA_TRY(cudaGetLastError());
-    int rc = launch_panel_syrk(reinterpret_cast<const double*>(workspace), chunks, n_red, 1, gram, s);
-    if (rc) return rc;
-  }
-  return AGF_OK;
+  return agf::gram_linear_ws_impl(forces, dtype, n_frames, n_sites, col_ptr, col_sites, n_red, gram, workspace,
+                                  workspace_bytes, nullptr, stream);
+}
+
+extern "C" int agf_gram_linear_ws_weighted(const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                                           const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red,
+                                           double* gram, void* workspace, size_t workspace_bytes,
+                                           const double* frame_weights, void* stream) {
+  return agf::gram_linear_ws_impl(forces, dtype, n_frames, n_sites, col_ptr, col_sites, n_red, gram, workspace,
+                                  workspace_bytes, frame_weights, stream);
 }
 
 extern "C" int agf_symmetrize(double* gram, int32_t n, void* stream) {

@@ -18,9 +18,12 @@ def constraint_aware_uni_map(
     traj: ForcesTrajectory,  # noqa: ARG001
     coord_map: LinearMap,
     constraints: Union[None, Constraints] = None,
+    frame_weights=None,  # noqa: ARG001
 ) -> SeperableTMap:
     """Each bead sums, unweighted, the forces of its own sites and of every site constrained
-    (transitively) to one of them.  ``traj`` is ignored."""
+    (transitively) to one of them.  ``traj`` is ignored, and so is ``frame_weights``: the map reads no
+    frames (it is accepted so that ``project_forces(..., frame_weights=w)`` reports the weighted residual
+    of this map too)."""
     matrix = np.asarray(coord_map.standard_matrix)
     try:  # pure index bookkeeping: memoised on the content of its two inputs (a fresh matrix per call)
         key = (matrix.shape, str(matrix.dtype), hashlib.blake2b(np.ascontiguousarray(matrix).tobytes(), digest_size=16).digest(),

@@ -268,14 +268,24 @@ class _FusedContext:
         return (p(self.d_grp_ptr), p(self.d_grp_sites), self.n_groups, self.n_channels, p(self.d_bead_ptr),
                 p(self.d_bead_sites), p(self.d_bead_w), self.n_cg, p(self.d_centers), self.nb, self.width, self.clip)
 
-    def grams(self, coords: _engine.Frames, forces: _engine.Frames, kbt: float, on_device: bool = False):
+    def grams(self, coords: _engine.Frames, forces: _engine.Frames, kbt: float, on_device: bool = False,
+              weights: Optional[torch.Tensor] = None):
         """All-reduced per-bead Grams in the user's feature order, ``(n_cg, n_feat, n_feat)`` float64
-        (numpy, or a CUDA tensor with ``on_device``)."""
+        (numpy, or a CUDA tensor with ``on_device``).  ``weights``: per-frame weights
+        (``_engine.frame_weights_dev``); weighted Grams run on the FP64 DMMA kernels only."""
         nf = self.n_feat_kernel
         gram = torch.zeros((self.n_cg, nf, nf), dtype=torch.float64, device=_engine.device())
-        for _, c, f in _engine.paired_pieces(coords, forces):
+        for t0, c, f in _engine.paired_pieces(coords, forces):
             if c.dtype != f.dtype:
                 c, f = c.to(torch.float64), f.to(torch.float64)
+            if weights is not None:
+                need = int(_lib.lib().agf_gram_feat_workspace_bytes(self.n_groups, self.n_channels, self.nb,
+                                                                    self.n_cg, c.shape[0]))
+                ws = _engine.workspace(need)
+                _lib.call("agf_gram_feat_ws_weighted", _engine.ptr(c), _engine.ptr(f), _engine.dtype_code(c),
+                          c.shape[0], self.n_fg, *self._common(), float(kbt), _engine.ptr(gram), _engine.ptr(ws),
+                          C.c_size_t(ws.numel()), _engine.ptr(weights[t0 : t0 + c.shape[0]]), _engine.stream_ptr())
+                continue
             need_i8 = 0
             if _engine._GRAM_I8[0] and nf > 97 and c.shape[0] >= _engine._GRAM_I8T_MIN_FRAMES:
                 need_i8 = int(_lib.lib().agf_gram_feat_i8_workspace_bytes(self.n_groups, self.n_channels, self.nb,
@@ -409,6 +419,7 @@ def qp_feat_linear_map(
     solver_args: SolverOptions = DEFAULT_SOLVER_OPTIONS,
     l2_regularization: float = 1e1,
     constraint_frames=None,
+    frame_weights=None,
 ) -> CLAFTMap:
     """Force map linear in user features, minimising the mean squared mapped force.
 
@@ -417,25 +428,32 @@ def qp_feat_linear_map(
     frame sum.  Extra keyword ``constraint_frames`` (array of frame indices, or callable
     ``(n_total, n) -> indices``) replaces the reference's unseeded random choice of the frames on
     which the bead-orthogonality constraints are imposed.
+
+    ``frame_weights`` (extension): one non-negative weight per frame (numpy or CUDA tensor; under
+    ``frame_sharding`` this rank's slice).  Every regression row of frame t (the ``kbt`` divergence term
+    included) is multiplied by ``sqrt(w_t)``, so ``P_c = sum_t w_t v_t v_t^T (+ l2 I)``.  The frames that
+    carry the equality rows are chosen as without weights: a constraint holds on a configuration whatever
+    its weight.
     """
     if constraints is None:
         constraints = set()
     warn_if_solver_ignored(solver_args)
+    weights = _engine.frame_weights_dev(frame_weights, traj.forces.shape[0])
     plan = _fusable(featurizer)
     if plan is not None:
         return _fit_fused(traj, coord_map, featurizer, plan, kbt, n_constraint_frames, constraints, solver_args,
-                          l2_regularization, constraint_frames)
+                          l2_regularization, constraint_frames, weights)
     return _fit_generic(traj, coord_map, featurizer, kbt, n_constraint_frames, constraints, sparse, solver_args,
-                        l2_regularization, constraint_frames)
+                        l2_regularization, constraint_frames, weights)
 
 
 def _fit_fused(traj, coord_map, featurizer, plan, kbt, n_constraint_frames, constraints, solver_args,
-               l2_regularization, constraint_frames) -> CLAFTMap:
+               l2_regularization, constraint_frames, weights=None) -> CLAFTMap:
     ctx = _FusedContext(coord_map, constraints, plan)
     coords, forces = _engine.Frames(traj.coords), _engine.Frames(traj.forces)
     backend = dict(solver_args or {}).get("backend", "exact")
     on_device = backend == "exact" and ctx.columns.size >= _DEVICE_SOLVE_MIN
-    grams = ctx.grams(coords, forces, kbt, on_device=on_device)  # large problems never leave the device
+    grams = ctx.grams(coords, forces, kbt, on_device=on_device, weights=weights)  # large problems never leave the device
     n_feat = grams.shape[1]
     coefs = []
     chosen = _ConstraintFrames(coords.n_frames, coord_map.n_cg_sites, n_constraint_frames, constraint_frames)
@@ -498,7 +516,7 @@ def _fit_fused(traj, coord_map, featurizer, plan, kbt, n_constraint_frames, cons
 
 
 def _fit_generic(traj, coord_map, featurizer, kbt, n_constraint_frames, constraints, sparse, solver_args,
-                 l2_regularization, constraint_frames) -> CLAFTMap:
+                 l2_regularization, constraint_frames, weights=None) -> CLAFTMap:
     dev = _engine.device()
     feat_results = featurizer(traj.coords, coord_map, constraints)
     feats, divs, names = (feat_results[k] for k in (KNAME_FEATS, KNAME_DIVS, KNAME_NAMES))
@@ -519,6 +537,8 @@ def _fit_generic(traj, coord_map, featurizer, kbt, n_constraint_frames, constrai
         target = np.zeros((len(frames), coord_map.n_cg_sites))
         target[:, bead] = 1
         rows = torch.einsum("tad,taf->tdf", forces, phi) + kbt * dv.transpose(1, 2)
+        if weights is not None:
+            rows = rows * weights.sqrt()[:, None, None]
         reg = rows.reshape(-1, rows.shape[2])
         gram = reg.T @ reg
         _engine.allreduce_sum_(gram)

@@ -67,12 +67,13 @@ def qp_form(target: np.ndarray) -> np.ndarray:
     return np.reshape(mixed, (mixed.shape[0] * mixed.shape[1], -1))
 
 
-def force_gram(forces, n_sites: int, constraints: Constraints):
+def force_gram(forces, n_sites: int, constraints: Constraints, weights=None):
     """``(gram (n_red, n_red) float64 on the host, columns)`` -- the QP objective of
-    ``qplinear.py:66-71``, accumulated on the GPU and all-reduced across frame shards."""
+    ``qplinear.py:66-71``, accumulated on the GPU and all-reduced across frame shards
+    (``weights``: per-frame weights from ``_engine.frame_weights_dev``)."""
     cols = reduced_columns(n_sites, constraints)
     n_red = int(cols.max()) + 1
-    gram = _engine.gram_linear(_engine.Frames(forces), cols, n_red)
+    gram = _engine.gram_linear(_engine.Frames(forces), cols, n_red, weights=weights)
     return _engine.to_host_overlapped(gram), cols
 
 
@@ -225,14 +226,14 @@ class _SmallFitPlan:
 
 
 def _fit_small_on_device(traj, coord_map: LinearMap, constraints, cols: np.ndarray, n_red: int, l2: float,
-                         solver_args) -> SeperableTMap:
+                         solver_args, weights=None) -> SeperableTMap:
     """Gram (kernel a) -> ``agf_qp_equality_small`` -> a ``LinearMap`` whose coefficients are already
     where kernel (d) reads them.  Nothing synchronises here when called through ``project_forces``
     (which reads status + coefficients once, after the applications); a direct call resolves the fit
     before returning, as the reference raises at fit time."""
     plan = _SmallFitPlan.get(coord_map, constraints, cols, n_red, l2)
     n_cg = plan.n_cg
-    gram, order = _engine.gram_linear_raw(_engine.Frames(traj.forces), cols, n_red, plan=plan.gram_plan)
+    gram, order = _engine.gram_linear_raw(_engine.Frames(traj.forces), cols, n_red, plan=plan.gram_plan, weights=weights)
     _engine.run_deferred()
     compiled = plan.compiled_structure.with_values(torch.empty((n_red, n_cg), dtype=torch.float64, device=gram.device))
     buf = torch.zeros(_DeviceFit.N_HEAD + n_cg * n_red, dtype=torch.float64, device=gram.device)
@@ -255,6 +256,7 @@ def qp_linear_map(
     constraints: Union[None, Constraints] = None,
     l2_regularization: float = 0.0,
     solver_args: SolverOptions = DEFAULT_SOLVER_OPTIONS,
+    frame_weights=None,
 ) -> SeperableTMap:
     """Linear force map minimising the mean squared mapped force.
 
@@ -266,6 +268,11 @@ def qp_linear_map(
     problem is solved exactly (closed form, on the device for small and for large reduced problems)
     unless ``solver_args={"backend": "qpsolvers", ...}``; other keys given without that backend are
     reported once with a warning and not used.
+
+    ``frame_weights`` (extension): one non-negative weight per frame (numpy or CUDA tensor; under
+    ``frame_sharding`` the weights of this rank's frames).  The objective becomes the raw weighted sum
+    ``P = sum_t w_t r_t r_t^T`` -- not normalised, so ``l2_regularization`` stays relative to that sum and
+    scaling both by ``c`` gives the same map.  Integer weights equal repeating frames.
     """
     if constraints is None:
         constraints = set()
@@ -273,6 +280,7 @@ def qp_linear_map(
     n_fg = coord_map.n_fg_sites
     if traj.forces.shape[1] != n_fg:
         raise ValueError("coord_map and forces disagree on the number of fine-grained sites.")
+    weights = _engine.frame_weights_dev(frame_weights, traj.forces.shape[0])
     backend = dict(solver_args or {}).get("backend", "exact")
     cols = reduced_columns(n_fg, constraints)
     n_red = int(cols.max()) + 1
@@ -280,12 +288,13 @@ def qp_linear_map(
     n_cg = coord_map.n_cg_sites
     if (backend == "exact" and not on_device and isinstance(coord_map, LinearMap)
             and _lib.lib().agf_qp_equality_small_supported(n_red, n_cg)):
-        return _fit_small_on_device(traj, coord_map, constraints, cols, n_red, l2_regularization, solver_args)
+        return _fit_small_on_device(traj, coord_map, constraints, cols, n_red, l2_regularization, solver_args,
+                                    weights)
     if on_device:
-        qp_mat = _engine.gram_linear(_engine.Frames(traj.forces), cols, n_red)  # stays on the device
+        qp_mat = _engine.gram_linear(_engine.Frames(traj.forces), cols, n_red, weights=weights)  # stays on the device
         _engine.run_deferred()
     else:
-        qp_mat, cols = force_gram(traj.forces, n_fg, constraints)
+        qp_mat, cols = force_gram(traj.forces, n_fg, constraints, weights)
     group_size = np.bincount(cols, minlength=n_red).astype(np.float64)
     if l2_regularization > 0.0:  # l2 * C'C
         if on_device:

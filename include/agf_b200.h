@@ -75,6 +75,22 @@ int agf_gram_linear_ws(const void* forces, int dtype, int64_t n_frames, int32_t 
                        const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red,
                        double* gram, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Per-frame weighted Gram  P += sum_t w_t v_t v_t^T  (weighted force-map fits: reweighted or pooled
+ * trajectories).  Same arguments, workspace and fallbacks as agf_gram_linear / agf_gram_linear_ws, plus
+ *   frame_weights  device f64 [n_frames], one weight per frame of THIS call (frame t of `forces` reads
+ *                  frame_weights[t]); the caller guarantees finite, non-negative values.  NULL = unweighted
+ *                  (identical to the entry points above).
+ * Runs the FP64 DMMA kernels: the group sums of frame t are multiplied by sqrt(w_t) in float64 where they
+ * are staged (n_red <= 128) or packed (n_red > 128).  The int8 tensor-core Grams have no weighted form.
+ */
+int agf_gram_linear_weighted(const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                             const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red,
+                             double* gram, const double* frame_weights, void* stream);
+int agf_gram_linear_ws_weighted(const void* forces, int dtype, int64_t n_frames, int32_t n_sites,
+                                const int32_t* col_ptr, const int32_t* col_sites, int32_t n_red,
+                                double* gram, void* workspace, size_t workspace_bytes,
+                                const double* frame_weights, void* stream);
+
 /* The same Gram through the 5th-generation tensor cores (tcgen05.mma kind::i8, accumulators in
  * TMEM): float32 forces, n_red <= 97, constraint groups of at most 4 sites.  Group sums are scaled per
  * column by a power of two taken from a sample of the frames, rounded to 39-bit fixed point and split
@@ -191,6 +207,15 @@ int agf_map_apply_slice(const void* points, int in_dtype, int64_t n_frames, int3
                         void* out, int out_dtype, double* sumsq, int nan_mode, double nan_atol,
                         int32_t* nan_flags, void* stream);
 
+/* Weighted residual numerator of a frame-weighted fit:  sumsq += sum_t w_t sum_e x[t, e]^2.
+ *   x              device [n_frames, per_frame] contiguous (a mapped array: per_frame = 3 n_cg), f32 or f64
+ *   frame_weights  device f64 [n_frames]
+ *   sumsq          device f64 [1] (+=)
+ * The unweighted sum comes from the `sumsq` epilogue of the agf_map_apply* kernels.
+ */
+int agf_weighted_sumsq(const void* x, int dtype, int64_t n_frames, int32_t per_frame,
+                       const double* frame_weights, double* sumsq, void* stream);
+
 /* ------------------------------------------------------------------------------------
  * (c) pair-distance moments for constraint detection.
  * Replaces  src/aggforce/util.py:64-70 (all-pairs displacement + norm) and
@@ -275,6 +300,26 @@ int agf_gram_feat_ws(const void* coords, const void* forces, int dtype, int64_t 
                      const int32_t* bead_sites, const double* bead_w, int32_t n_cg,
                      const double* centers, int32_t nb, double width, double clip, double kbt,
                      double* gram, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Per-frame weighted featurised Grams  P_c += sum_t w_t v_t v_t^T: every regression row of frame t
+ * (id and gb columns, the kbt divergence term included) is multiplied by sqrt(w_t) in float64 once it
+ * is complete.  Same arguments, workspace and fallbacks as agf_gram_feat / agf_gram_feat_ws, plus
+ *   frame_weights  device f64 [n_frames], one finite non-negative weight per frame of this call; NULL =
+ *                  unweighted.  FP64 DMMA kernels only (no weighted form of agf_gram_feat_i8).
+ */
+int agf_gram_feat_weighted(const void* coords, const void* forces, int dtype, int64_t n_frames,
+                           int32_t n_sites, const int32_t* grp_ptr, const int32_t* grp_sites,
+                           int32_t n_groups, int32_t n_channels, const int32_t* bead_ptr,
+                           const int32_t* bead_sites, const double* bead_w, int32_t n_cg,
+                           const double* centers, int32_t nb, double width, double clip, double kbt,
+                           double* gram, const double* frame_weights, void* stream);
+int agf_gram_feat_ws_weighted(const void* coords, const void* forces, int dtype, int64_t n_frames,
+                              int32_t n_sites, const int32_t* grp_ptr, const int32_t* grp_sites,
+                              int32_t n_groups, int32_t n_channels, const int32_t* bead_ptr,
+                              const int32_t* bead_sites, const double* bead_w, int32_t n_cg,
+                              const double* centers, int32_t nb, double width, double clip, double kbt,
+                              double* gram, void* workspace, size_t workspace_bytes,
+                              const double* frame_weights, void* stream);
 
 /* The featurised Gram on the 5th-generation tensor cores (n_feat > 97; float32 or float64 input): same contract and
  * arguments as agf_gram_feat_ws.  The regression rows are evaluated in float64 exactly as there, scaled per
