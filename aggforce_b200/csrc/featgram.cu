@@ -840,7 +840,9 @@ static int gram_feat_ws_impl(const void* coords, const void* forces, int dtype, 
                           bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, frame_weights, stream);
   AGF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) % 16) == 0, "agf_gram_feat_ws: workspace must be 16-byte aligned");
   if (n_frames == 0) return AGF_OK;
-  if (pack_smem > (size_t)200 * 1024)  // > 3200 constraint groups: per-frame records do not fit in shared memory
+  // feat_pack_kernel keeps one 8-double record per (frame, group) for kPanelKF = 8 frames in shared memory,
+  // 512 bytes per group: above 400 constraint groups they exceed 200 KiB and the fused kernel runs instead
+  if (pack_smem > (size_t)200 * 1024)
     return gram_feat_impl(coords, forces, dtype, n_frames, n_sites, grp_ptr, grp_sites, n_groups, n_channels, bead_ptr,
                           bead_sites, bead_w, n_cg, centers, nb, width, clip, kbt, gram, frame_weights, stream);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);

@@ -544,6 +544,106 @@ def feat_map_apply(
     return out
 
 
+# Group-level restatement of the featurised path (SURVEY 8a, A11).  Both feature families are one-hot in the
+# site's constraint group, so the contraction over sites collapses to group force sums and group mean
+# positions; these functions never materialise the (T, n_sites, n_feat) feature tensor of ``gb_features`` and
+# so reach shapes where that tensor would take gigabytes.  ``labels[a]`` is the group of site a (any order of
+# the groups); the first ``n_channels`` groups carry Gaussian channels (G or G-1: Q5).
+def _group_geometry(coords, cmap_row, labels, centers, width, clip, n_channels):
+    """Per frame and group: size m, mean position, distance d and unit vector to the bead, and the clipped
+    Gaussians g_k(d) with their derivative g_k'(d) for the first n_channels groups (float64)."""
+    x = np.asarray(coords, dtype=np.float64)
+    lab = np.asarray(labels, dtype=np.int64)
+    n_groups = int(lab.max()) + 1
+    m = np.bincount(lab, minlength=n_groups).astype(np.float64)
+    pos = np.zeros((x.shape[0], n_groups, 3))
+    for g in range(n_groups):
+        pos[:, g] = x[:, lab == g].sum(1) / m[g]
+    w = np.asarray(cmap_row, dtype=np.float64)
+    nz = np.nonzero(w)[0]
+    bead = np.einsum("k,tkd->td", w[nz], x[:, nz])
+    disp = pos[:, :n_channels] - bead[:, None, :]
+    dist = np.sqrt((disp * disp).sum(-1))
+    with np.errstate(invalid="ignore", divide="ignore"):
+        unit = disp / dist[..., None]  # NaN where a group mean sits on the bead (Q6)
+    z = (dist[..., None] - np.asarray(centers, dtype=np.float64)) / width
+    e = np.exp(-(z * z))
+    g = np.maximum(e, clip) - clip
+    gp = np.where(e > clip, -2.0 * z / width * e, 0.0)
+    return m, dist, unit, g, gp
+
+
+def _group_sums(values, labels, n_groups):
+    v = np.asarray(values, dtype=np.float64)
+    lab = np.asarray(labels, dtype=np.int64)
+    out = np.zeros((v.shape[0], n_groups, 3))
+    for g in range(n_groups):
+        out[:, g] = v[:, lab == g].sum(1)
+    return out
+
+
+def feat_group_rows(coords, forces, cmap_matrix, labels, bead, centers, width, clip, n_channels, kbt) -> np.ndarray:
+    """Regression rows of one bead, ``(3T, G + nb * n_channels)`` ordered (frame, dim) like
+    ``feat_regressor_rows`` on ``id_features`` + ``gb_features(div_method="basic")``:
+    ``v[g] = Fg[t,g,d]`` and ``v[G + ch*nb + k] = g_k(d_ch) Fg[t,ch,d] + kbt m_ch g_k'(d_ch) u_ch[d]``."""
+    lab = np.asarray(labels, dtype=np.int64)
+    n_groups = int(lab.max()) + 1
+    nb = len(centers)
+    m, _, unit, g, gp = _group_geometry(coords, np.asarray(cmap_matrix)[bead], lab, centers, width, clip, n_channels)
+    fg = _group_sums(forces, lab, n_groups)
+    gb = g[..., None] * fg[:, :n_channels, None, :] + kbt * m[:n_channels, None, None] * gp[..., None] * unit[:, :, None, :]
+    rows = np.concatenate([fg, gb.reshape(fg.shape[0], n_channels * nb, 3)], axis=1)  # (T, n_feat, 3)
+    return np.swapaxes(rows, 1, 2).reshape(-1, rows.shape[1])
+
+
+def feat_group_constraint_rows(coords, cmap_matrix, labels, bead, frame_indices, centers, width, clip,
+                               n_channels) -> np.ndarray:
+    """Equality rows of one bead, ``(n_sel * n_cg, n_feat)``, as ``feat_constraint_rows`` on ``id_features`` +
+    ``gb_features``: row (s, c') is ``sum_a cmap[c', a] phi[t_s, a, :]`` with ``phi`` one-hot in the group."""
+    lab = np.asarray(labels, dtype=np.int64)
+    cm = np.asarray(cmap_matrix, dtype=np.float64)
+    n_groups, nb = int(lab.max()) + 1, len(centers)
+    x = np.asarray(coords)[np.asarray(frame_indices)]
+    _, _, _, g, _ = _group_geometry(x, cm[bead], lab, centers, width, clip, n_channels)
+    # weight of each group in each bead row: sum of the bead's site weights in that group
+    gw = np.zeros((cm.shape[0], n_groups))
+    for a in np.nonzero(cm.any(0))[0]:
+        gw[:, lab[a]] += cm[:, a]
+    ids = np.broadcast_to(gw, (x.shape[0],) + gw.shape)
+    gb = gw[None, :, :n_channels, None] * g[:, None, :, :]  # (n_sel, n_cg, n_ch, nb)
+    rows = np.concatenate([ids, gb.reshape(x.shape[0], cm.shape[0], n_channels * nb)], axis=2)
+    return rows.reshape(-1, rows.shape[2])
+
+
+def feat_group_apply(coords, forces, cmap_matrix, labels, coefs, centers, width, clip, n_channels,
+                     magnitude: bool = False) -> np.ndarray:
+    """Mapped forces ``(T, n_cg, 3)`` of a fitted featurised map, as ``feat_map_apply`` on ``id_features`` +
+    ``gb_features``: ``sum_g (c[g] + sum_k c[G+g*nb+k] g_k(d_g)) Fg + sum_{g,k} c[G+g*nb+k] m_g g_k'(d_g) u_g``
+    (no kbt: Q7).  ``magnitude=True`` evaluates the same sum with every term by its absolute value and the
+    group forces as sums of |F|: the scale of the rounding error of any evaluation order."""
+    lab = np.asarray(labels, dtype=np.int64)
+    cm = np.asarray(cmap_matrix, dtype=np.float64)
+    co = np.asarray(coefs, dtype=np.float64)
+    n_groups, nb = int(lab.max()) + 1, len(centers)
+    f = np.asarray(forces, dtype=np.float64)
+    fg = _group_sums(np.abs(f) if magnitude else f, lab, n_groups)
+    ab = np.abs if magnitude else (lambda v: v)
+    out = np.zeros((f.shape[0], cm.shape[0], 3))
+    for c in range(cm.shape[0]):
+        m, _, unit, g, gp = _group_geometry(coords, cm[c], lab, centers, width, clip, n_channels)
+        cg = co[c, n_groups:].reshape(n_channels, nb)
+        w = np.broadcast_to(ab(co[c, :n_groups]), (f.shape[0], n_groups)).copy()
+        w[:, :n_channels] += (ab(cg[None] * g)).sum(-1)
+        tr = m[:n_channels] * ab(cg[None] * gp).sum(-1)  # (T, n_ch)
+        out[:, c] = np.einsum("tg,tgd->td", w, fg)
+        if n_channels:
+            out[:, c] += (tr[..., None] * ab(unit)).sum(1)
+    return out
+
+
+__all__ += ["feat_group_rows", "feat_group_constraint_rows", "feat_group_apply"]
+
+
 # --------------------------------------------------------------------------------------
 # config 5: Gaussian augmentation with injected noise
 # --------------------------------------------------------------------------------------

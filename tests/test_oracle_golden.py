@@ -185,6 +185,106 @@ def test_gb_divergence_against_finite_differences():
     assert np.allclose(mu, 8 * np.arange(7) ** 2 / 36.0)
 
 
+def _group_system(seed, sizes, n_frames, n_cg=3):
+    """Constraint groups of the given sizes over shuffled sites, weighted multi-site bead rows (one site in
+    two beads), coordinates spread over 0..12 from the beads."""
+    rng = np.random.default_rng(seed)
+    n = int(sum(sizes))
+    perm = rng.permutation(n)
+    groups = np.split(perm, np.cumsum(sizes)[:-1])
+    cons = {frozenset(int(v) for v in p) for g in groups for p in zip(g[:-1], g[1:])}
+    labels = oracle.canonical_labels(n, cons)
+    cm = np.zeros((n_cg, n))
+    for c in range(n_cg):
+        sites = rng.choice(n, size=int(rng.integers(2, 7)), replace=False)
+        cm[c, sites] = rng.uniform(0.2, 1.0, size=sites.size)
+    cm[1, np.nonzero(cm[0])[0][0]] = 0.7  # a site shared by two beads
+    cm /= cm.sum(1, keepdims=True)
+    centres = rng.uniform(-5.0, 5.0, size=(n_frames, len(sizes), 3))
+    x = np.empty((n_frames, n, 3))
+    for g, members in enumerate(groups):
+        x[:, members] = centres[:, g, None, :] + rng.normal(0.0, 0.4, size=(n_frames, members.size, 3))
+    return x, rng.normal(0.0, 5.0, size=(n_frames, n, 3)), cm, cons, labels
+
+
+GROUP_SIZES = [1, 3, 12, 2, 5, 1, 4, 2, 1, 7]
+
+
+@pytest.mark.parametrize("drop", [True, False])
+def test_feat_group_rows_match_the_literal_restatement(drop):
+    """The group-level rows equal id_features + gb_features("basic") + feat_regressor_rows, and the group-level
+    equality rows equal feat_constraint_rows, on weighted multi-site beads and groups of 1 to 12 sites."""
+    x, f, cm, cons, labels = _group_system(5, GROUP_SIZES, 6)
+    kw = dict(outer=8.0, inner=0.0, n_basis=5, width=0.8, clip=1e-3)
+    mu = oracle.gb_centers(0.0, 8.0, 5)
+    n_groups = int(labels.max()) + 1
+    n_ch = n_groups - 1 if drop else n_groups
+    idf, idd = oracle.id_features(len(x), labels)
+    frames = [4, 0, 4, 2]
+    for bead in range(cm.shape[0]):
+        gf, gd = oracle.gb_features(x, cm, cons, labels, bead, drop_last_channel=drop, div_method="basic", **kw)
+        feats, divs = np.concatenate([idf, gf], axis=2), np.concatenate([idd, gd], axis=1)
+        want = oracle.feat_regressor_rows(f, feats, divs, 0.7)
+        got = oracle.feat_group_rows(x, f, cm, labels, bead, mu, 0.8, 1e-3, n_ch, 0.7)
+        assert got.shape == want.shape == (3 * len(x), n_groups + 5 * n_ch)
+        assert np.all(np.abs(got - want) <= 1e-13 * np.maximum(1.0, np.abs(want)))
+        a_ref, _ = oracle.feat_constraint_rows(feats, cm, bead, frames)
+        a = oracle.feat_group_constraint_rows(x, cm, labels, bead, frames, mu, 0.8, 1e-3, n_ch)
+        assert a.shape == a_ref.shape and np.all(np.abs(a - a_ref) <= 1e-13 * np.maximum(1.0, np.abs(a_ref)))
+    # id features only (n_channels = 0)
+    got = oracle.feat_group_rows(x, f, cm, labels, 0, mu, 0.8, 1e-3, 0, 0.7)
+    assert np.abs(got - oracle.feat_regressor_rows(f, idf, idd, 0.7)).max() <= 1e-13 * np.abs(f).sum(1).max()
+
+
+@pytest.mark.parametrize("drop", [True, False])
+def test_feat_group_apply_matches_feat_map_apply(drop):
+    x, f, cm, cons, labels = _group_system(6, GROUP_SIZES, 5)
+    kw = dict(outer=8.0, inner=0.0, n_basis=4, width=1.0, clip=1e-3)
+    mu = oracle.gb_centers(0.0, 8.0, 4)
+    n_groups = int(labels.max()) + 1
+    n_ch = n_groups - 1 if drop else n_groups
+    idf, idd = oracle.id_features(len(x), labels)
+    coefs = np.random.default_rng(1).normal(size=(cm.shape[0], n_groups + 4 * n_ch))
+    feats, divs = [], []
+    for bead in range(cm.shape[0]):
+        gf, gd = oracle.gb_features(x, cm, cons, labels, bead, drop_last_channel=drop, div_method="basic", **kw)
+        feats.append(np.concatenate([idf, gf], axis=2))
+        divs.append(np.concatenate([idd, gd], axis=1))
+    want = oracle.feat_map_apply(f, feats, divs, coefs)
+    got = oracle.feat_group_apply(x, f, cm, labels, coefs, mu, 1.0, 1e-3, n_ch)
+    scale = oracle.feat_group_apply(x, f, cm, labels, coefs, mu, 1.0, 1e-3, n_ch, magnitude=True)
+    assert got.shape == want.shape and np.all(np.abs(got - want) <= 1e-13 * scale)
+    assert np.all(scale >= np.abs(want))
+    got0 = oracle.feat_group_apply(x, f, cm, labels, coefs[:, :n_groups], mu, 1.0, 1e-3, 0)
+    want0 = oracle.feat_map_apply(f, [idf] * cm.shape[0], [idd] * cm.shape[0], coefs[:, :n_groups])
+    assert np.all(np.abs(got0 - want0) <= 1e-13 * np.abs(want0).max())
+
+
+def test_feat_group_functions_keep_the_basic_nan_pattern():
+    """A one-site group on a slice bead (SURVEY Q6): NaN in that group's channel only, as gb_features "basic",
+    and a NaN mapped force for that bead."""
+    x, f, cm, cons, labels = _group_system(7, GROUP_SIZES, 4)
+    site = int(np.nonzero(np.bincount(labels)[labels] == 1)[0][0])
+    cm[0] = 0.0
+    cm[0, site] = 1.0
+    ch = int(labels[site])
+    kw = dict(outer=8.0, inner=0.0, n_basis=3, width=1.0, clip=1e-3)
+    mu = oracle.gb_centers(0.0, 8.0, 3)
+    n_groups = int(labels.max()) + 1
+    gf, gd = oracle.gb_features(x, cm, cons, labels, 0, drop_last_channel=False, div_method="basic", **kw)
+    idf, idd = oracle.id_features(len(x), labels)
+    want = oracle.feat_regressor_rows(f, np.concatenate([idf, gf], axis=2), np.concatenate([idd, gd], axis=1), 0.7)
+    got = oracle.feat_group_rows(x, f, cm, labels, 0, mu, 1.0, 1e-3, n_groups, 0.7)
+    nan_cols = np.isnan(got).any(0)
+    assert np.array_equal(np.isnan(got), np.isnan(want))
+    assert np.array_equal(np.nonzero(nan_cols)[0], n_groups + 3 * ch + np.arange(3))
+    ok = ~np.isnan(want)
+    assert np.all(np.abs(got[ok] - want[ok]) <= 1e-13 * np.maximum(1.0, np.abs(want[ok])))
+    coefs = np.random.default_rng(2).normal(size=(cm.shape[0], n_groups + 3 * n_groups))
+    out = oracle.feat_group_apply(x, f, cm, labels, coefs, mu, 1.0, 1e-3, n_groups)
+    assert np.isnan(out[:, 0]).all() and np.isfinite(out[:, 1:]).all()
+
+
 def test_condnormal_closed_form(golden):
     ref = np.load(golden / "ref_condnormal.npz")
     var = float(ref["var"])
