@@ -37,7 +37,9 @@ inline ChunkSchedule make_schedule(const void* base, int64_t n_frames, int64_t f
   int head = 0;
   uintptr_t a = reinterpret_cast<uintptr_t>(base);
   while (head < 16 && head < n_frames && ((a + (uintptr_t)head * (uintptr_t)frame_bytes) % 16) != 0) ++head;
-  if (head >= 16) head = (int)(n_frames < kf ? n_frames : kf);  // hopeless alignment: everything cooperative
+  // hopeless alignment: everything cooperative.  With fewer than 16 frames the search also ends at n_frames, which
+  // may be more frames than a chunk (a stage) holds.
+  if (head >= 16 || head > kf) head = (int)(n_frames < kf ? n_frames : kf);
   s.head = head;
   int64_t rest = n_frames - head;
   s.n_chunks = 1 + (rest + kf - 1) / kf;

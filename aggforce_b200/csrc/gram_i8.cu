@@ -192,6 +192,11 @@ __global__ void __launch_bounds__(kI8Threads, 1) gram_i8_kernel(const __grid_con
     // Fixed point in ONE instruction: t = fma(v, 2^(39-E), 1.5 * 2^52 + B) holds q + B in its low 40 bits
     // (round to nearest), and its upper 24 bits are a known constant exactly when |q| is in range.
     const int n_quads = p.n_red > kI8N ? kI8N / 4 + 1 : kI8N / 4;
+    // The first member is loaded without a mask.  A column with no sites (empty, or past n_red) keeps scale 0, so
+    // the value it loads gives digit 0, and it loads the first listed site: a non-finite value there sends the
+    // frame to the float64 pass whatever this column does.  (With the exponent of an all-zero column, -900, any
+    // non-zero value would leave the fixed-point range and the frame would be added in float64 for nothing.)
+    const uint32_t idle_off = s_ptr[p.n_red] > 0 ? (uint32_t)s_sites[0] * 12u : 0u;
     uint32_t moff[4][4];
     float mask[4][4];
     double scale[4];
@@ -201,7 +206,7 @@ __global__ void __launch_bounds__(kI8Threads, 1) gram_i8_kernel(const __grid_con
       scale[cc] = 0.0;
 #pragma unroll
       for (int m = 0; m < 4; ++m) {
-        moff[cc][m] = 0;
+        moff[cc][m] = m == 0 ? idle_off : 0u;
         mask[cc][m] = 0.f;
       }
       if (lane < n_quads && x < p.n_red) {
@@ -213,7 +218,7 @@ __global__ void __launch_bounds__(kI8Threads, 1) gram_i8_kernel(const __grid_con
             moff[cc][m] = (uint32_t)s_sites[b + m] * 12u;
             mask[cc][m] = 1.f;
           }
-        scale[cc] = ldexp(1.0, 39 - s_exp[x]);
+        if (n > 0) scale[cc] = ldexp(1.0, 39 - s_exp[x]);
       }
     }
     const double magic = 6755399441055744.0 + 551911719040.0;  // 1.5 * 2^52 + 0x8080808080

@@ -21,6 +21,7 @@ __all__ = [
     "group_columns",
     "bond_constraint_matrix",
     "gram_linear",
+    "gram_csr",
     "l2_linear_term",
     "solve_equality_qp",
     "qp_linear_weights",
@@ -205,6 +206,29 @@ def gram_linear(forces: np.ndarray, constraints: Iterable[Iterable[int]] = ()) -
     cmat = bond_constraint_matrix(n_sites, constraints)
     reg = f.transpose(0, 2, 1).reshape(n_frames * n_dim, n_sites) @ cmat
     return reg.T @ reg
+
+
+def gram_csr(forces: np.ndarray, col_ptr: np.ndarray, col_sites: np.ndarray,
+             weights: Optional[np.ndarray] = None) -> np.ndarray:
+    """``sum_t w_t v_t v_t^T`` in float64 for any column table of the C ABI: column x sums the forces of the sites
+    ``col_sites[col_ptr[x]:col_ptr[x + 1]]``.  Sites may be in no column, columns may be empty and come in any
+    order; rows are the (frame, xyz) pairs of :func:`gram_linear`.  ``weights`` (one per frame) scale each frame's
+    contribution; ``None`` means 1."""
+    f = np.asarray(forces, dtype=np.float64)
+    ptr_ = np.asarray(col_ptr, dtype=np.int64)
+    sites = np.asarray(col_sites, dtype=np.int64)
+    n_frames = f.shape[0]
+    n_red = ptr_.size - 1
+    # sums over each column's members only (not a product with a 0/1 matrix): a non-finite force of a site in no
+    # column must not reach any column
+    reg = np.zeros((n_frames, 3, n_red))
+    for x in range(n_red):
+        reg[:, :, x] = f[:, sites[ptr_[x] : ptr_[x + 1]], :].sum(axis=1)
+    reg = reg.reshape(n_frames * 3, n_red)
+    if weights is not None:
+        reg = reg * np.repeat(np.sqrt(np.asarray(weights, dtype=np.float64)), 3)[:, None]
+    # einsum's own loops, not BLAS: every product is formed, so NaN and Inf propagate as IEEE arithmetic says
+    return np.einsum("ri,rj->ij", reg, reg)
 
 
 def l2_linear_term(n_sites: int, constraints: Iterable[Iterable[int]] = ()) -> np.ndarray:

@@ -70,6 +70,62 @@ def test_gram_linear_matches_reference(small_cln):
     assert p.shape == (97, 97)
 
 
+def _csr_of_columns(cols, n_red):
+    """(col_ptr, col_sites) of a site -> column table (-1: in no column)."""
+    ptr = np.zeros(n_red + 1, dtype=np.int64)
+    ptr[1:] = np.cumsum(np.bincount(cols[cols >= 0], minlength=n_red))
+    return ptr, np.argsort(np.where(cols >= 0, cols, n_red), kind="stable")[: ptr[-1]]
+
+
+def _assert_close_per_element(got, ref, tol):
+    d = np.sqrt(np.diag(ref))
+    assert np.all(np.abs(got - ref) <= tol * d[:, None] * d[None, :])
+
+
+def test_gram_csr_matches_gram_linear(small_cln):
+    """gram_csr on the column table of the constraint groups is gram_linear; unweighted, weighted against frames
+    scaled by sqrt(w) (a zero and a 1e3 weight among them), and with the columns in another order."""
+    forces = small_cln["forces"]
+    cons = pairs_to_set(small_cln["cons10"])
+    cols = oracle.group_columns(forces.shape[1], cons)
+    n_red = int(cols.max()) + 1
+    ptr, sites = _csr_of_columns(cols, n_red)
+    ref = oracle.gram_linear(forces, cons)
+    _assert_close_per_element(oracle.gram_csr(forces, ptr, sites), ref, 1e-13)
+    w = np.random.default_rng(0).uniform(0.5, 2.0, size=forces.shape[0])
+    w[0], w[5] = 0.0, 1e3
+    scaled = forces.astype(np.float64) * np.sqrt(w)[:, None, None]
+    ref_w = oracle.gram_linear(scaled, cons)
+    _assert_close_per_element(oracle.gram_csr(forces, ptr, sites, w), ref_w, 1e-13)
+    _assert_close_per_element(oracle.gram_csr(scaled, ptr, sites), ref_w, 1e-13)
+    perm = np.random.default_rng(1).permutation(n_red)  # column x of the new table is column perm[x] of the old
+    rank = np.empty(n_red, dtype=np.int64)
+    rank[perm] = np.arange(n_red)
+    pptr, psites = _csr_of_columns(rank[cols], n_red)
+    _assert_close_per_element(oracle.gram_csr(forces, pptr, psites), ref[np.ix_(perm, perm)], 1e-13)
+
+
+def test_gram_csr_sites_in_no_column_and_empty_columns(small_cln):
+    """Sites in no column do not reach the Gram, even when their forces are not finite; an empty column is an
+    exactly zero row and column; the other elements are the Gram of the columns that remain."""
+    forces = small_cln["forces"].astype(np.float64)
+    cons = pairs_to_set(small_cln["cons10"])
+    cols = oracle.group_columns(forces.shape[1], cons)
+    n_red = int(cols.max()) + 1
+    ref = oracle.gram_linear(forces, cons)
+    gone = np.nonzero(cols == 7)[0]           # column 7 loses all its sites: it stays, empty
+    cols2 = np.where(cols == 7, -1, cols)
+    ptr, sites = _csr_of_columns(cols2, n_red)
+    assert ptr[8] == ptr[7]
+    poisoned = forces.copy()
+    poisoned[0, gone[0]] = np.nan
+    poisoned[1, gone[-1]] = np.inf
+    got = oracle.gram_csr(poisoned, ptr, sites)
+    assert np.all(got[7] == 0) and np.all(got[:, 7] == 0)
+    keep = np.arange(n_red) != 7
+    _assert_close_per_element(got[np.ix_(keep, keep)], ref[np.ix_(keep, keep)], 1e-13)
+
+
 def test_linear_weights_match_reference(small_cln):
     from aggforce_b200.synth import chignolin_topology
 
